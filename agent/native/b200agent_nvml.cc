@@ -15,6 +15,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <time.h>
 
 #include <mutex>
 #include <vector>
@@ -58,6 +59,7 @@ struct Api {
 #define X(n) decltype(&::n) n = nullptr;
   NVML_FUNCS(X)
 #undef X
+  decltype(&::nvmlDeviceGetUtilizationRates) nvmlDeviceGetUtilizationRates = nullptr;   // optional: the sampler's fallback
   void* handle = nullptr;
   bool ok = false;
   char why[256] = {0};
@@ -87,6 +89,7 @@ void load_api() {
   if (!g_api.n) { all = false; snprintf(g_api.why, sizeof(g_api.why), "libnvidia-ml lacks %s", #n); }
   NVML_FUNCS(X)
 #undef X
+  g_api.nvmlDeviceGetUtilizationRates = reinterpret_cast<decltype(g_api.nvmlDeviceGetUtilizationRates)>(dlsym(g_api.handle, "nvmlDeviceGetUtilizationRates"));
   g_api.ok = all;
 }
 
@@ -97,6 +100,24 @@ int need_api() {
 }
 
 struct EventSet { nvmlEventSet_t set; };
+
+// Some drivers refuse the utilisation sample buffer with NOT_SUPPORTED (580.178 on a B200 sizes it, then will not fill it). The
+// driver's utilisation rate is then the one sample there is: the share of its last sample period (1/6 s to 1 s) in which a kernel
+// ran, read now. It is newer than any cut-off in the past and there is none newer than a cut-off in the future.
+int utilization_rate(nvmlDevice_t d, unsigned long long since_us, unsigned int* util, nvmlReturn_t refused, const char* what) {
+  if (!g_api.nvmlDeviceGetUtilizationRates) { set_err(what, refused); return (int)refused; }
+  timespec now;
+  clock_gettime(CLOCK_REALTIME, &now);
+  if (since_us > (unsigned long long)now.tv_sec * 1000000ull + (unsigned long long)now.tv_nsec / 1000) {
+    snprintf(g_last_error, sizeof(g_last_error), "no utilisation samples newer than the cut-off");
+    return B200NVML_NO_SAMPLES;
+  }
+  nvmlUtilization_t u;
+  nvmlReturn_t r = g_api.nvmlDeviceGetUtilizationRates(d, &u);
+  if (r != NVML_SUCCESS) { set_err("nvmlDeviceGetUtilizationRates", r); return (int)r; }
+  *util = u.gpu;
+  return B200NVML_OK;
+}
 
 }  // namespace
 
@@ -170,10 +191,12 @@ int b200nvml_average_usage(const char* uuid, unsigned long long since_us, unsign
   nvmlValueType_t vt;
   unsigned int count = 0;
   r = g_api.nvmlDeviceGetSamples(d, NVML_GPU_UTILIZATION_SAMPLES, since_us, &vt, &count, nullptr);   // size query
+  if (r == NVML_ERROR_NOT_SUPPORTED) return utilization_rate(d, since_us, util, r, "nvmlDeviceGetSamples(size)");
   if (r != NVML_SUCCESS) { set_err("nvmlDeviceGetSamples(size)", r); return (int)r; }
   if (count == 0) { snprintf(g_last_error, sizeof(g_last_error), "no utilisation samples newer than the cut-off"); return B200NVML_NO_SAMPLES; }
   std::vector<nvmlSample_t> samples(count);
   r = g_api.nvmlDeviceGetSamples(d, NVML_GPU_UTILIZATION_SAMPLES, since_us, &vt, &count, samples.data());
+  if (r == NVML_ERROR_NOT_SUPPORTED) return utilization_rate(d, since_us, util, r, "nvmlDeviceGetSamples");
   if (r != NVML_SUCCESS) { set_err("nvmlDeviceGetSamples", r); return (int)r; }
   if (count == 0) return B200NVML_NO_SAMPLES;
   unsigned long long sum = 0;

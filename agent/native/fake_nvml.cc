@@ -2,7 +2,9 @@
 // above it (discovery, duty-cycle sampler, Xid health loop) run end to end on a GPU-less CI box.
 // Scripted by environment: FAKE_NVML_GPUS (count, default 2), FAKE_NVML_UTIL ("50,60,70" sample values,
 // empty = no samples), FAKE_NVML_EVENTS (file with "gpu_index xid [gi ci]" lines; each Wait pops one line,
-// "-1 xid" = event without a device), FAKE_NVML_NO_EVENTS=1 (RegisterEvents returns NOT_SUPPORTED).
+// "-1 xid" = event without a device), FAKE_NVML_NO_EVENTS=1 (RegisterEvents returns NOT_SUPPORTED),
+// FAKE_NVML_SAMPLES_UNSUPPORTED=1 (GetSamples sizes the buffer but refuses to fill it, as some drivers do; GetUtilizationRates
+// then reports the last FAKE_NVML_UTIL value).
 #include "nvml_abi.h"
 #include <stdio.h>
 #include <stdlib.h>
@@ -53,14 +55,23 @@ nvmlReturn_t nvmlDeviceGetMemoryInfo(nvmlDevice_t, nvmlMemory_t* m) { m->total =
 nvmlReturn_t nvmlDeviceGetMigMode(nvmlDevice_t, unsigned int* c, unsigned int* p) { *c = *p = getenv("FAKE_NVML_MIG") ? 1 : 0; return NVML_SUCCESS; }
 nvmlReturn_t nvmlSystemGetDriverVersion(char* buf, unsigned int len) { const char* v = getenv("FAKE_NVML_DRIVER"); snprintf(buf, len, "%s", v ? v : "580.159.03"); return NVML_SUCCESS; }
 nvmlReturn_t nvmlDeviceGetSupportedEventTypes(nvmlDevice_t, unsigned long long* t) { *t = nvmlEventTypeXidCriticalError; return NVML_SUCCESS; }
-nvmlReturn_t nvmlDeviceGetSamples(nvmlDevice_t, nvmlSamplingType_t, unsigned long long, nvmlValueType_t* vt, unsigned int* count, nvmlSample_t* samples) {
+static unsigned util_values(unsigned* vals) {
   const char* e = getenv("FAKE_NVML_UTIL");
-  unsigned vals[128]; unsigned n = 0;
+  unsigned n = 0;
   if (e) { const char* p = e; while (*p && n < 128) { vals[n++] = (unsigned)strtoul(p, (char**)&p, 10); if (*p == ',') p++; else break; } }
   else { vals[0] = 40; vals[1] = 60; n = 2; }
-  if (e && !*e) n = 0;
+  return e && !*e ? 0 : n;
+}
+nvmlReturn_t nvmlDeviceGetUtilizationRates(nvmlDevice_t, nvmlUtilization_t* u) {
+  unsigned vals[128]; unsigned n = util_values(vals);
+  u->gpu = n ? vals[n - 1] : 0; u->memory = 0;
+  return NVML_SUCCESS;
+}
+nvmlReturn_t nvmlDeviceGetSamples(nvmlDevice_t, nvmlSamplingType_t, unsigned long long, nvmlValueType_t* vt, unsigned int* count, nvmlSample_t* samples) {
+  unsigned vals[128]; unsigned n = util_values(vals);
   *vt = NVML_VALUE_TYPE_UNSIGNED_INT;
   if (!samples) { *count = n; return NVML_SUCCESS; }
+  if (getenv("FAKE_NVML_SAMPLES_UNSUPPORTED")) return NVML_ERROR_NOT_SUPPORTED;
   if (*count > n) *count = n;
   for (unsigned i = 0; i < *count; i++) { samples[i].timeStamp = 1; samples[i].sampleValue.uiVal = vals[i]; }
   return NVML_SUCCESS;

@@ -10,7 +10,13 @@ A "step" is one pass over the 21-size sweep (1 KB..1 GB, x2), out-of-place and i
 reference's nccl-tests protocol each size's `--steps` iterations are launched back to back and timed with
 CUDA events on the launching stream (after `--warmup` untimed launches), bracketed by a cross-rank barrier
 and torch.cuda.synchronize(); every number is the max over ranks. `value` is nccl-tests' "Avg bus bandwidth".
-Rank 0 prints ONE JSON line.
+The end-to-end sweep (host in, host out) runs `--steps` steps as well. Rank 0 prints ONE JSON line.
+
+The send buffer is filled from a seeded hash before the sweep, so the same arguments give the same inputs on
+every run (harness.fill_inputs says why the receive buffer is not). `--dump-outputs DIR` makes rank 0
+write what the last timed step of every size returned, as DIR/<op>_<oop|ip|e2e>_<bytes>B.npy in float32:
+whole outputs when small, otherwise a fixed sample of their elements (first and last ones included), at
+most 64 MiB in all. Two builds run with the same arguments can then be compared output for output.
 """
 from __future__ import annotations
 
@@ -23,16 +29,57 @@ import time
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 
+DUMP_LIMIT = 64 << 20      # bytes of .npy payload --dump-outputs may write, all arrays together
+
+
 def parse_size(s: str) -> int:
     s = s.strip().upper()
     mult = {"K": 1 << 10, "M": 1 << 20, "G": 1 << 30}
     return int(float(s[:-1]) * mult[s[-1]]) if s[-1] in mult else int(s)
 
 
+def positive_int(s: str) -> int:
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
+class OutputDump:
+    """Collects the outputs handed to harness.sweep's on_output as float32 copies: whole when they hold at most `per_array` elements,
+    otherwise the first and last 1024 elements plus one element from each of `per_array - 2048` equal stretches in between, at an
+    offset given by a hash of the stretch's number. The sample depends on the output's length only, so two runs with the same
+    arguments sample the same elements. Copies of device outputs stay on the device until write(): the capture between two timed
+    windows is a few kernel launches on the sweep's stream, with no host synchronisation and no idle GPU."""
+
+    def __init__(self, n_arrays: int):
+        self.per_array = max(4096, DUMP_LIMIT // 4 // max(1, n_arrays))
+        self.arrays = {}
+
+    def __call__(self, name: str, t) -> None:
+        import torch
+        n = t.numel()
+        if n > self.per_array:
+            edge, k = 1024, self.per_array - 2048
+            span = n - 2 * edge
+            j = torch.arange(k, device=t.device)
+            mid = edge + j * span // k + (((j * 2654435761) & 0xFFFFFFFF) >> 8) % (span // k)
+            t = t[torch.cat([torch.arange(edge, device=t.device), mid, torch.arange(n - edge, n, device=t.device)])]
+        self.arrays[name] = t.to(torch.float32, copy=True)
+
+    def write(self, out_dir: str) -> None:
+        import numpy as np
+        total = sum(a.numel() * 4 for a in self.arrays.values())
+        assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}"
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in self.arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def main() -> int:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference-sym"], help="reference = stock NCCL on plain buffers (what nccl-tests does); reference-sym = the same on ncclMemAlloc memory with symmetric windows registered (NCCL's own fast path)")
     ap.add_argument("--op", default="all_reduce", choices=["all_reduce", "all_gather", "reduce_scatter", "alltoall", "broadcast", "reduce", "sendrecv", "gather", "scatter"])
@@ -42,6 +89,7 @@ def main() -> int:
     ap.add_argument("--table", action="store_true", help="also print the nccl-tests style table to stderr")
     ap.add_argument("--extra-ops", default="", help="comma list of further collectives to sweep in the same process group; results go to --extra-out, never to stdout")
     ap.add_argument("--extra-out", default="gpurun_out/extra_ops.json")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of every size returned to DIR/<name>.npy (float32, at most 64 MiB in all)")
     args = ap.parse_args()
     warmup = max(3, args.warmup)
 
@@ -81,10 +129,15 @@ def main() -> int:
 
     n = dist.world
     verified = harness.verify(backend, dist, args.op, dtype)
+    harness.fill_inputs(backend, dist)
+    dump = None
+    if args.dump_outputs and dist.rank == 0:
+        n_sizes = sum(1 for k in range(64) if min_b << k <= max_b)
+        dump = OutputDump(3 * n_sizes)          # at most out-of-place, in-place and end-to-end per size
     launches0 = backend.launches()
     t_wall = time.time()
     with ClockSampler(dist.local_rank) as clk:
-        rows = harness.sweep(backend, dist, args.op, dtype, args.steps, warmup, min_b, max_b, placements=(0, 1))
+        rows = harness.sweep(backend, dist, args.op, dtype, args.steps, warmup, min_b, max_b, placements=(0, 1), on_output=dump)
     launches = backend.launches() - launches0
     clocks = clk.summary()
     e2e = None
@@ -92,8 +145,8 @@ def main() -> int:
     if not args.no_e2e:
         e2e_ok = harness.verify_e2e(backend, dist, dtype) if args.op == "all_reduce" else True
         hl0 = backend.launches()
-        e2e_steps = max(2, min(args.steps, 10))
-        e2e_rows = harness.sweep(backend, dist, args.op, dtype, e2e_steps, min(warmup, 3), min_b, max_b, placements=(), e2e=True)
+        e2e_steps = args.steps
+        e2e_rows = harness.sweep(backend, dist, args.op, dtype, e2e_steps, min(warmup, 3), min_b, max_b, placements=(), e2e=True, on_output=dump)
         s2 = harness.summarize(e2e_rows, args.op, n)
         e2e = {"value": round(s2["avg_e2e_busbw"] or 0.0, 3), "unit": "GB/s", "h2d_bytes_per_step": int(sum(r.in_bytes for r in e2e_rows)),
                "d2h_bytes_per_step": int(sum(r.out_bytes for r in e2e_rows)), "steps": e2e_steps, "verified_vs_torch_fp32": bool(e2e_ok),
@@ -135,6 +188,8 @@ def main() -> int:
                                      "(net plugins are off the intra-node path), so this arm is the image's stock libnccl called through its C API with the "
                                      "NCCL's own defaults (B200_REF_PROFILE=1 applies the reference's multi-node env profile, gpudirect-tcpxo/README.md:71-103); pip install of /root/reference: see DESIGN.md")
         print(json.dumps(out), flush=True)
+    if dump is not None:
+        dump.write(args.dump_outputs)
     if args.extra_ops:
         extra = {}
         for op in [o for o in args.extra_ops.split(",") if o and o != args.op]:

@@ -49,7 +49,7 @@ class Node:
     def __init__(self, command: str, gpus: int = 2, mig_parts: int = 0, config=None, numa=None, extra: str = "", env=None, kubelet: bool = True, real: bool = False):
         """real=True: no fakes on the device side — the host's /dev, /proc, /sys and the installed libnvidia-ml (tests/test_agent_gpu.py,
         run on a GPU box); the kubelet is still the stub."""
-        self.tmp = tempfile.TemporaryDirectory(prefix="b200-conformance-")
+        self.tmp = tempfile.TemporaryDirectory(prefix="b200-conformance-", dir=testing.socket_tmp_root())
         root = self.tmp.name
         self.real = real
         self.plugin_dir = os.path.join(root, "device-plugins"); os.makedirs(self.plugin_dir)
@@ -336,7 +336,7 @@ def metrics_endpoint(cmd):
     import urllib.request
     from concurrent import futures
     from container_engine_accelerators_b200.agent import protos
-    with tempfile.TemporaryDirectory() as d:
+    with tempfile.TemporaryDirectory(dir=testing.socket_tmp_root()) as d:
         pr = protos.podresources
         resp = pr.ListPodResourcesResponse()
         for ns, pod, ctr, ids in (("default", "trainer-0", "main", ["nvidia0"]), ("default", "shared-1", "main", ["nvidia1/vgpu0"])):

@@ -6,6 +6,7 @@ language-neutral harness: anything that speaks v1beta1 over a Unix socket can be
 from __future__ import annotations
 
 import os
+import tempfile
 import threading
 from concurrent import futures
 from pathlib import Path
@@ -14,6 +15,17 @@ import grpc
 
 from . import protos
 from .protos import deviceplugin as pb
+
+# A Unix socket's address holds at most 107 bytes, and the fakes and plugins bind theirs inside temporary directories (the longest
+# name used is "device-plugins/nvidiaGPU-conformance.sock"). A directory path no longer than SOCKET_DIR_MAX leaves room for it.
+SOCKET_DIR_MAX = 64
+
+
+def socket_tmp_root() -> str:
+    """Where to create temporary directories that will hold Unix sockets: the usual temporary directory when its path takes at most half
+    of SOCKET_DIR_MAX (the rest is for the directory made inside it), otherwise /tmp."""
+    base = tempfile.gettempdir()
+    return base if len(base) <= SOCKET_DIR_MAX // 2 else "/tmp"
 
 
 class KubeletStub:

@@ -415,8 +415,24 @@ def verify_e2e(backend, dist: Dist, dtype) -> bool:
     return dist.sum_([1.0 if ok else 0.0])[0] == dist.world
 
 
+def fill_inputs(backend, dist: Dist, chunk: int = 1 << 26) -> None:
+    """Seeded contents for the whole send buffer (same integer hash as verify()), so that what a sweep computes depends on its
+    arguments only. The receive buffer is left as allocated: the out-of-place pass writes it before anything reads it, and the in-place
+    pass reads what the out-of-place pass of the same size wrote. Writing it here would also slow the timed copies into it: on a B200,
+    sizes of 256 KB - 8 MB (which fit in L2) took 6.3 instead of 4.6 us per launch once the receive buffer had been written before."""
+    import torch
+    gen = _gen_expected(torch, "all_reduce", dist.rank, dist.world, 0, None)
+    buf = backend.send
+    for lo in range(0, buf.numel(), chunk):
+        hi = min(lo + chunk, buf.numel())
+        buf[lo:hi] = gen(dist.rank, torch.arange(lo, hi, device=buf.device)).to(buf.dtype)
+    torch.cuda.synchronize()
+
+
 def sweep(backend, dist: Dist, op: str, dtype, steps: int, warmup: int, min_bytes: int, max_bytes: int, factor: int = 2,
-          placements=(0, 1), e2e: bool = False) -> list[Row]:
+          placements=(0, 1), e2e: bool = False, on_output=None) -> list[Row]:
+    """on_output(name, tensor), when given, is called after each timed window (outside it) with what the window's last launch wrote:
+    the output in the device receive buffer, or for e2e the whole pinned host result."""
     import torch
     n, rank = dist.world, dist.rank
     itemsize = backend.send.element_size()
@@ -481,6 +497,10 @@ def sweep(backend, dist: Dist, op: str, dtype, steps: int, warmup: int, min_byte
             e1.record(stream)
             torch.cuda.synchronize()
             raw.append((len(rows), "ip" if ip else "oop", e0.elapsed_time(e1) / steps))
+            if on_output is not None:
+                r = ptrs((steps - 1) % slots)[1]
+                lo = (r - rbase) // itemsize
+                on_output(f"{op}_{'ip' if ip else 'oop'}_{total:010d}B", backend.recv[lo:lo + out_elems])
         if e2e:
             # the user-visible step: this rank's input starts in pinned host memory and the whole result ends there
             h_in, h_out = host_in[:in_elems], host_out[:out_elems]
@@ -495,6 +515,8 @@ def sweep(backend, dist: Dist, op: str, dtype, steps: int, warmup: int, min_byte
             e1.record(stream)
             torch.cuda.synchronize()
             raw.append((len(rows), "e2e", e0.elapsed_time(e1) / steps))
+            if on_output is not None:
+                on_output(f"{op}_e2e_{total:010d}B", h_out)
         rows.append(row)
         nbytes *= factor
     backend.check()

@@ -1,7 +1,10 @@
 """pytest configuration: registers the `gpu` marker and builds native artefacts once per session."""
 import os
+import pathlib
+import shutil
 import subprocess
 import sys
+import tempfile
 
 import pytest
 
@@ -11,6 +14,19 @@ sys.path.insert(0, ROOT)
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with `pytest -m gpu` on the GPU box)")
+
+
+@pytest.fixture
+def tmp_path(tmp_path):
+    """pytest's tmp_path, or a shorter directory when that one is too deep for the Unix sockets the agent tests bind in it (a long
+    TMPDIR, user name or --basetemp would otherwise fail them with "AF_UNIX path too long")."""
+    from container_engine_accelerators_b200.agent import testing
+    if len(str(tmp_path)) <= testing.SOCKET_DIR_MAX:
+        yield tmp_path
+        return
+    short = tempfile.mkdtemp(prefix="b200-test-", dir=testing.socket_tmp_root())
+    yield pathlib.Path(short)
+    shutil.rmtree(short, ignore_errors=True)
 
 
 @pytest.fixture(scope="session")

@@ -170,30 +170,11 @@ def test_driver_version_annotations_preserve_others():
 
 
 # ------------------------------------------------------------------------------------------------- wire schemas vs upstream .proto files
-def _parse_proto(path):
-    """Minimal .proto reader: {message: {field name: (number, type, repeated)}} — enough to compare names, numbers, types and cardinality."""
-    import re
-    text = re.sub(r"//[^\n]*", "", open(path).read())
-    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-    text = re.sub(r"\[[^\]]*\]", "", text)                       # field options such as (gogoproto.customname)
-    out, stack = {}, []
-    for tok in re.finditer(r"message\s+(\w+)\s*\{|enum\s+(\w+)\s*\{|oneof\s+\w+\s*\{|\}|(repeated\s+|optional\s+)?(map\s*<\s*\w+\s*,\s*[\w.]+\s*>|[\w.]+)\s+(\w+)\s*=\s*(\d+)\s*;", text):
-        if tok.group(1):
-            stack.append(tok.group(1)); out.setdefault(tok.group(1), {})
-        elif tok.group(2):
-            stack.append("enum:" + tok.group(2)); out.setdefault("__enums__", set()).add(tok.group(2))
-        elif tok.group(0).startswith("oneof"):
-            stack.append("oneof")
-        elif tok.group(0) == "}":
-            if stack:
-                stack.pop()
-        else:
-            owner = next((s for s in reversed(stack) if not s.startswith("enum:") and s != "oneof"), None)
-            if owner is None or (stack and stack[-1].startswith("enum:")):
-                continue
-            typ = re.sub(r"\s+", "", tok.group(4))
-            out[owner][tok.group(5)] = (int(tok.group(6)), typ.split(".")[-1] if not typ.startswith("map<") else typ, bool(tok.group(3) and tok.group(3).strip() == "repeated"))
-    return out
+# What the upstream sources say is stored in tests/golden/reference_facts.json (oracle/reference_facts.py regenerates it), so these
+# comparisons run everywhere, not only next to an upstream checkout.
+def _reference_facts(section):
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_facts.json")) as f:
+        return json.load(f)[section]
 
 
 _SCALARS = {9: "string", 8: "bool", 3: "int64", 5: "int32", 13: "uint32", 4: "uint64", 12: "bytes", 1: "double", 2: "float"}
@@ -221,10 +202,9 @@ def test_kubelet_schemas_match_the_upstream_proto_files(ours, upstream):
     """protos.py builds descriptors at run time from a hand-written table (the image has no protoc); every message and field in that
     table must agree — name, number, type, repeated — with the schema the kubelet is compiled from. Fields we do not model are fine
     (proto3 skips unknown fields); a wrong number or type is not."""
-    path = os.path.join("/root/reference/vendor", upstream)
-    if not os.path.exists(path):
-        pytest.skip("upstream .proto not available")
-    theirs = _parse_proto(path)
+    assert _reference_facts("proto_sources")[ours].endswith(upstream)
+    theirs = {name: {f: tuple(spec) for f, spec in fields.items()} if name != "__enums__" else set(fields)
+              for name, fields in _reference_facts("proto_schemas")[ours].items()}
     ns = getattr(protos, ours)
     checked = 0
     for name, cls in vars(ns).items():
@@ -245,39 +225,29 @@ def test_contract_constants_match_the_reference_sources():
     """Names that other systems key on (Prometheus queries, node-problem-detector, the kubelet, job templates) must be the reference's
     exactly, in the Python agent AND in the native binary: monitored Xids, gauge names, annotation keys, condition / event strings,
     resource name, topology labels, NRI annotation prefix."""
-    import re
-    ref = "/root/reference"
-    if not os.path.exists(ref):
-        pytest.skip("reference not available")
     from container_engine_accelerators_b200.agent import health, metrics, nri as nrimod
     from container_engine_accelerators_b200.scheduler import topology as topo
+    ref = _reference_facts("contract_constants")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     native = open(os.path.join(root, "agent", "native", "dp", "device_plugin.cc")).read()
-    hc = open(f"{ref}/pkg/gpu/nvidia/health_check/health_checker.go").read()
-    xids = tuple(int(x) for x in re.search(r"monitorCriticalXid := \[\]int\{([^}]*)\}", hc).group(1).split(","))
+    xids = tuple(ref["monitor_xids"])
     assert health.MONITOR_XIDS == xids and "kMonitorXids[] = {" + ", ".join(map(str, xids)) + "}" in native
-    assert 'Type:               "XidCriticalError"' in hc or '"XidCriticalError"' in hc
+    assert ref["xid_condition_type"] == "XidCriticalError"
     assert health.XID_CONDITION_TYPE == "XidCriticalError" and 'kXidCondition = "XidCriticalError"' in native
-    assert '"nvidia-gpu-device-plugin"' in hc and health.EVENT_SOURCE == "nvidia-gpu-device-plugin" and 'kEventSource = "nvidia-gpu-device-plugin"' in native
-    gauges = re.findall(r'Name: "(\w+)"', open(f"{ref}/pkg/gpu/nvidia/metrics/metrics.go").read())
+    assert ref["event_source"] == "nvidia-gpu-device-plugin" and health.EVENT_SOURCE == "nvidia-gpu-device-plugin" and 'kEventSource = "nvidia-gpu-device-plugin"' in native
+    gauges = ref["gauges"]
     assert sorted(gauges) == sorted(["duty_cycle_gpu_node", "memory_total_gpu_node", "memory_used_gpu_node", "duty_cycle", "memory_total", "memory_used", "request"])
     ours = {m._name for m in metrics.MetricServer(nvml.MockNvml("/nonexistent"))._all}
     assert set(gauges) <= ours
     for g in gauges:
         assert f'"{g}"' in native or f'"{g.replace("_gpu_node", "")}"' in native, g
-    vv = open(f"{ref}/pkg/gpu/nvidia/version_visibility/version_visibility.go").read()
-    prefix = re.search(r'DriverVersionPrefix\s*=\s*"([^"]+)"', vv).group(1)
+    prefix = ref["driver_version_prefix"]
     assert version_visibility.PREFIX == prefix + "." and f'"{prefix}."' in native
-    assert 'FieldManager: "gpu-device-plugin"' in vv or '"gpu-device-plugin"' in vv
+    assert ref["field_manager"] == "gpu-device-plugin"
     assert version_visibility.FIELD_MANAGER == "gpu-device-plugin" and '"gpu-device-plugin"' in native
-    assert 'resourceName = "nvidia.com/gpu"' in open(f"{ref}/pkg/gpu/nvidia/manager.go").read().replace("\t", " ").replace("  ", " ") or "nvidia.com/gpu" in open(f"{ref}/pkg/gpu/nvidia/manager.go").read()
+    assert ref["resource_name"] == "nvidia.com/gpu"
     assert mgr.RESOURCE_NAME == "nvidia.com/gpu" and 'kResourceName = "nvidia.com/gpu"' in native
-    sched = open(f"{ref}/gke-topology-scheduler/schedule-daemon.py").read()
-    labels = dict(re.findall(r"^(\w+_LABEL) = '([^']+)'", sched, re.M))
-    assert topo.PRERELEASE_LABELS == (labels["PRERELEASE_CLUSTER_LABEL"], labels["PRERELEASE_RACK_LABEL"], labels["PRERELEASE_HOST_LABEL"])
-    assert topo.GA_LABELS == (labels["CLUSTER_LABEL"], labels["RACK_LABEL"], labels["HOST_LABEL"])
-    inj = open(f"{ref}/nri_device_injector/nri_device_injector.go").read()
-    key = re.search(r'ctrDeviceKeyPrefix\s*=\s*"([^"]+)"', inj)
-    if key:
-        assert nrimod.CTR_DEVICE_KEY_PREFIX == key.group(1)
+    assert topo.PRERELEASE_LABELS == tuple(ref["topology_labels"]["prerelease"])
+    assert topo.GA_LABELS == tuple(ref["topology_labels"]["ga"])
+    assert nrimod.CTR_DEVICE_KEY_PREFIX == ref["nri_container_device_key_prefix"]
     assert nrimod.CTR_DEVICE_KEY_PREFIX == "devices.gke.io/container." and "devices.gke.io/container." in open(os.path.join(root, "agent", "native", "dp", "nri_injector.cc")).read()

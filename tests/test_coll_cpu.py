@@ -181,7 +181,12 @@ def test_nccl_shim_exports_the_api_nccl_tests_links_against(coll_lib):
             "ncclCommRevoke", "ncclGroupSimulateEnd"}
     # and nothing the installed NCCL header declares is missing from the shim
     import re
-    hdr = next((p for p in ("/opt/prime-rl/.venv/lib/python3.12/site-packages/nvidia/nccl/include/nccl.h", "/usr/include/nccl.h") if os.path.exists(p)), None)
+    try:                                                           # the header of the NCCL wheel that torch runs on, else the system one
+        import nvidia.nccl
+        wheel = [os.path.join(d, "include", "nccl.h") for d in nvidia.nccl.__path__]
+    except ImportError:
+        wheel = []
+    hdr = next((p for p in wheel + ["/usr/include/nccl.h"] if os.path.exists(p)), None)
     if hdr:
         declared = set(re.findall(r"^\s*(?:ncclResult_t|const char\*)\s+(nccl[A-Za-z]+)\s*\(", open(hdr).read(), re.M))
         assert declared <= syms, sorted(declared - syms)
@@ -195,6 +200,32 @@ def test_nccl_shim_exports_the_api_nccl_tests_links_against(coll_lib):
         comms = (C.c_void_p * 1)()
         rc = L.ncclCommInitAll(comms, 1, (C.c_int * 1)(0))
         assert rc != 0 and L.ncclGetErrorString(rc)               # no driver: an error code, not a crash
+
+
+def test_bench_output_dump_samples_the_same_elements_within_budget(tmp_path):
+    """bench.py --dump-outputs: small outputs whole; large ones reduced to a sample that depends on their length only (so two builds
+    dump the same elements), sorted, without repeats, with the first and last 1024 elements; float32 .npy files within 64 MiB."""
+    import importlib.util
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_main", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"))
+    bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
+    runs = []
+    for _ in range(2):
+        d = bench.OutputDump(63)
+        d("small", torch.arange(256, dtype=torch.bfloat16))
+        for n in (d.per_array + 1, 10_000_019):
+            d(f"n{n}", torch.arange(n, dtype=torch.float32))           # exact in float32 below 2**24: the values are the sampled indices
+        d.write(str(tmp_path / f"run{len(runs)}"))
+        runs.append({p.stem: np.load(p) for p in (tmp_path / f"run{len(runs)}").glob("*.npy")})
+    assert runs[0].keys() == runs[1].keys() == {"small", f"n{d.per_array + 1}", "n10000019"}
+    assert all(np.array_equal(runs[0][k], runs[1][k]) and runs[0][k].dtype == np.float32 for k in runs[0])
+    assert np.array_equal(runs[0]["small"], np.arange(256, dtype=np.float32))
+    for n in (d.per_array + 1, 10_000_019):
+        idx = runs[0][f"n{n}"].astype(np.int64)
+        assert len(idx) == d.per_array and (np.diff(idx) > 0).all() and idx.min() == 0 and idx.max() == n - 1
+        assert np.array_equal(idx[:1024], np.arange(1024)) and np.array_equal(idx[-1024:], np.arange(n - 1024, n))
+    assert d.per_array * 4 * 63 <= bench.DUMP_LIMIT
 
 
 def test_harness_bandwidth_accounting_follows_nccl_tests():

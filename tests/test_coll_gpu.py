@@ -398,9 +398,12 @@ def test_multi_gpu_procs_nvls(torch_cuda, coll_lib):
         assert r.returncode == 0 and "errors=0" in r.stdout, r.stdout + r.stderr
 
 
-def test_bench_contract_one_gpu(torch_cuda):
+def test_bench_contract_one_gpu(torch_cuda, tmp_path):
     import json
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--max", "16M"], capture_output=True, text=True, timeout=300)
+    import numpy as np
+    dump = tmp_path / "outputs"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--max", "16M", "--dump-outputs", str(dump)],
+                       capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr
     line = [l for l in r.stdout.splitlines() if l.startswith("{")]
     assert len(line) == 1
@@ -412,6 +415,14 @@ def test_bench_contract_one_gpu(torch_cuda):
     assert d["verified_vs_torch_fp32"] is True and d["e2e"]["verified_vs_torch_fp32"] is True
     assert len(d["e2e"]["table"]) == len(d["table"]) and all(r["e2e_us"] > 0 for r in d["e2e"]["table"])      # per-size end-to-end rows are published
     assert d["impl"] == "ours" and d["backend"].startswith("libb200coll") and "backend" not in d["config"]   # config is identical on both arms
+    assert d["steps"] == 3 and d["e2e"]["steps"] == 3                                  # --steps sets the timed steps of both sweeps
+    arrays = {p.stem: np.load(p) for p in dump.glob("*.npy")}
+    assert set(arrays) == {f"all_reduce_{k}_{1024 << i:010d}B" for k in ("oop", "e2e") for i in range(15)}    # 1K..16M, one rank: no in-place pass
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in arrays.values()) and sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    assert all((a == 0.25).all() for k, a in arrays.items() if "_e2e_" in k)              # host input 0.25 everywhere, one rank: the sum is the input
+    elems = {k: int(k.split("_")[-1][:-1]) // 2 for k in arrays}
+    sample = max(a.size for a in arrays.values())
+    assert sample < elems["all_reduce_oop_0016777216B"] and all(a.size == min(elems[k], sample) for k, a in arrays.items())   # small outputs whole, large ones sampled
 
 
 

@@ -297,6 +297,24 @@ h = n.events_open(); print("reg", n.events_register(h, 0))
     assert "code -5" in r.stdout and "reg False" in r.stdout          # reference divides by sampleCount == 0 here (util.go:82)
 
 
+def test_native_sampler_falls_back_when_the_driver_refuses_samples(native):
+    """Some drivers size the utilisation sample buffer, then refuse to fill it (NOT_SUPPORTED). The duty cycle is then the driver's
+    utilisation rate over its last sample period; a cut-off in the future still has no sample."""
+    code = """
+import time
+from container_engine_accelerators_b200.agent import nvml
+n = nvml.NativeNvml(); n.init()
+print("util", n.average_usage("GPU-fake-0", int((time.time() - 10) * 1e6)))
+try:
+    n.average_usage("GPU-fake-0", int((time.time() + 3600) * 1e6)); print("no-error")
+except nvml.NvmlError as e:
+    print("future", e.code)
+"""
+    r = run_py(code, {"FAKE_NVML_UTIL": "40,60,95", "FAKE_NVML_SAMPLES_UNSUPPORTED": "1"})
+    assert r.returncode == 0, r.stderr
+    assert "util 95" in r.stdout and "future -5" in r.stdout, r.stdout
+
+
 def test_native_without_nvml_library_reports_cleanly(native_build):
     code = """
 from container_engine_accelerators_b200.agent import nvml

@@ -273,16 +273,13 @@ def test_native_json_agrees_with_python_on_generated_documents(native_build):
 
 def test_mig_table_covers_every_size_the_reference_knows():
     """mig_profiles.inc is the single table behind the plugin and the partitioner; every (size -> profile id, max count) the reference
-    lists in its two tables (partition_gpu.go:37-139, pkg/gpu/nvidia/mig/mig.go:35-82) must be there with the same numbers."""
+    lists in its two tables (partition_gpu.go:37-139, pkg/gpu/nvidia/mig/mig.go:35-82) must be there with the same numbers. The
+    reference's tables are recorded in tests/golden/reference_facts.json (oracle/reference_facts.py)."""
     import re
-    ref = "/root/reference/partition_gpu/partition_gpu.go"
-    if not os.path.exists(ref):
-        pytest.skip("reference not available")
-    go = open(ref).read()
-    ids = dict(re.findall(r'"(\d+g\.\d+gb)":\s*"(\d+)"', go[go.index("partitionSizeToProfileID"):go.index("partitionSizeMaxCount")]))
-    counts = dict(re.findall(r'"(\d+g\.\d+gb)":\s*(\d+),', go[go.index("partitionSizeMaxCount"):]))
-    plugin_counts = dict(re.findall(r'"(\d+g\.\d+gb)":\s*(\d+),', open("/root/reference/pkg/gpu/nvidia/mig/mig.go").read()))
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    with open(os.path.join(root, "tests", "golden", "reference_facts.json")) as f:
+        tables = json.load(f)["mig_tables"]
+    ids, counts, plugin_counts = tables["partition_profile_ids"], tables["partition_max_counts"], tables["plugin_max_counts"]
     ours = {m.group(1): (m.group(2), m.group(3)) for m in re.finditer(r'MIG_PROFILE\("([\w.]+)",\s*(\d+),\s*(\d+),', open(os.path.join(root, "agent", "native", "mig_profiles.inc")).read())}
     assert len(ids) >= 20 and set(ids) <= set(ours), sorted(set(ids) - set(ours))
     for size, pid in ids.items():

@@ -222,19 +222,15 @@ def test_python_injector_as_a_process(tmp_path):
 def test_wire_constants_match_the_vendored_containerd_sources():
     """Our two NRI stacks are tested against our own fake runtime; pin the framing constants to containerd's sources so that
     agreement is not just self-consistency: ttrpc header 10 bytes / request 1 / response 2, mux header 8 bytes, conn ids 1 and 2,
-    CREATE_CONTAINER = 4 (event mask bit 3)."""
-    import re
-    base = "/root/reference/vendor/github.com/containerd"
-    if not os.path.exists(base):
-        pytest.skip("vendored containerd sources not available")
-    chan = open(f"{base}/ttrpc/channel.go").read()
-    assert re.search(r"messageHeaderLength\s*=\s*10", chan) and re.search(r"messageTypeRequest\s+messageType\s*=\s*0x1", chan) and re.search(r"messageTypeResponse\s+messageType\s*=\s*0x2", chan)
-    mux = open(f"{base}/nri/pkg/net/multiplex/mux.go").read()
-    assert re.search(r"headerLen\s*=\s*8", mux) and re.search(r"maxPayloadSize\s*=\s*1\s*<<\s*24", mux) and "binary.BigEndian.PutUint32(hdr[0:4], uint32(id))" in mux
-    ids = open(f"{base}/nri/pkg/net/multiplex/ttrpc.go").read()
-    assert re.search(r"PluginServiceConn ConnID = iota \+ 1\s*\n\s*//[^\n]*\n\s*RuntimeServiceConn", ids)
-    api = open(f"{base}/nri/pkg/api/api.proto").read()
-    assert re.search(r"CREATE_CONTAINER\s*=\s*4\s*;", api)
-    assert (nri.PLUGIN_SERVICE_CONN, nri.RUNTIME_SERVICE_CONN) == (1, 2) and protos.NRI_EVENT_CREATE_CONTAINER == 1 << 3
+    CREATE_CONTAINER = 4 (event mask bit 3). The vendored sources' values are recorded in tests/golden/reference_facts.json
+    (oracle/reference_facts.py)."""
+    import json
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_facts.json")) as f:
+        wire = json.load(f)["containerd_wire"]
+    assert (wire["ttrpc_header_bytes"], wire["ttrpc_request_type"], wire["ttrpc_response_type"]) == (10, 1, 2)
+    assert (wire["mux_header_bytes"], wire["mux_max_payload_bytes"]) == (8, 1 << 24) and wire["mux_conn_id_big_endian_at_0"] is True
+    assert (wire["plugin_service_conn"], wire["runtime_service_conn"]) == (1, 2)
+    assert wire["create_container_event"] == 4
+    assert (nri.PLUGIN_SERVICE_CONN, nri.RUNTIME_SERVICE_CONN) == (1, 2) and protos.NRI_EVENT_CREATE_CONTAINER == 1 << wire["create_container_event"] - 1
     native = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "agent", "native", "dp", "nri_injector.cc")).read()
     assert "kPluginConn = 1, kRuntimeConn = 2" in native and "kRequest = 1, kResponse = 2" in native and "pb::put_int(&resp, 2, 1 << 3)" in native
