@@ -50,7 +50,7 @@ typedef enum {
   b200collFloat32 = 0,
   b200collFloat16 = 1,
   b200collBfloat16 = 2,
-  b200collFloat8e4m3 = 3,   /* output / wire type only */
+  b200collFloat8e4m3 = 3,   /* fp8 e4m3 (OCP "fn": max 448): input and output type */
   /* the types below take the generic reduction path (src/generic.cu): same type in and out, no scale, any operator but avg */
   b200collInt8 = 4,
   b200collUint8 = 5,
@@ -59,11 +59,16 @@ typedef enum {
   b200collInt64 = 8,
   b200collUint64 = 9,
   b200collFloat64 = 10,
-  b200collNumTypes = 11
+  /* fp8 e5m2 (max 57344): input and output type, like e4m3 */
+  b200collFloat8e5m2 = 11,
+  b200collNumTypes = 12
 } b200collDataType_t;
 
-/* sum and avg of fp16 / bf16 / fp32 run on the fused fast paths (Lamport, two-shot, NVLS); prod, min, max — and every operator on the
- * integer types and fp64 — run on one barrier-based P2P kernel that accumulates in the element type. */
+/* sum and avg of fp32 / fp16 / bf16 / fp8 e4m3 / fp8 e5m2 run on the fused fast paths (Lamport, two-shot, NVLS) and accumulate in fp32;
+ * fp8 results are rounded to nearest and saturate to the largest finite value. prod, min, max — and every operator on the integer types
+ * and fp64 — run on one barrier-based P2P kernel that accumulates in the element type (fp16 / bf16 / fp8 in fp32).
+ * Supported (in_dtype, out_dtype) pairs: equal types; fp32 <-> bf16 / fp16 widen or narrow; fp32 / bf16 / fp16 -> e4m3 or e5m2
+ * (quantise); e4m3 or e5m2 -> bf16 / fp16 / fp32 (dequantise, with the fused scale). There is no e4m3 <-> e5m2 pair. */
 typedef enum { b200collSum = 0, b200collAvg = 1, b200collProd = 2, b200collMin = 3, b200collMax = 4 } b200collRedOp_t;
 
 typedef enum {

@@ -18,8 +18,10 @@ namespace b200coll {
 template <typename T> struct Tag { using type = T; };
 using bf16 = __nv_bfloat16;
 using f8 = __nv_fp8_e4m3;
+using f8e5 = __nv_fp8_e5m2;
 
-// Supported (in, out) pairs: same type, widen to f32, narrow f32 to 16-bit, quantise to e4m3.
+// Supported (in, out) pairs: same type, widen to f32, narrow f32 to 16-bit, quantise to e4m3 / e5m2, dequantise fp8 to a wider
+// type (no cross-fp8 pair).
 template <typename F>
 static b200collResult_t dispatch_types(b200collDataType_t in, b200collDataType_t out, F&& f) {
   if (in == b200collFloat32) {
@@ -28,6 +30,7 @@ static b200collResult_t dispatch_types(b200collDataType_t in, b200collDataType_t
       case b200collBfloat16: return f(Tag<float>{}, Tag<bf16>{});
       case b200collFloat16: return f(Tag<float>{}, Tag<__half>{});
       case b200collFloat8e4m3: return f(Tag<float>{}, Tag<f8>{});
+      case b200collFloat8e5m2: return f(Tag<float>{}, Tag<f8e5>{});
       default: break;
     }
   } else if (in == b200collBfloat16) {
@@ -35,6 +38,7 @@ static b200collResult_t dispatch_types(b200collDataType_t in, b200collDataType_t
       case b200collBfloat16: return f(Tag<bf16>{}, Tag<bf16>{});
       case b200collFloat32: return f(Tag<bf16>{}, Tag<float>{});
       case b200collFloat8e4m3: return f(Tag<bf16>{}, Tag<f8>{});
+      case b200collFloat8e5m2: return f(Tag<bf16>{}, Tag<f8e5>{});
       default: break;
     }
   } else if (in == b200collFloat16) {
@@ -42,12 +46,36 @@ static b200collResult_t dispatch_types(b200collDataType_t in, b200collDataType_t
       case b200collFloat16: return f(Tag<__half>{}, Tag<__half>{});
       case b200collFloat32: return f(Tag<__half>{}, Tag<float>{});
       case b200collFloat8e4m3: return f(Tag<__half>{}, Tag<f8>{});
+      case b200collFloat8e5m2: return f(Tag<__half>{}, Tag<f8e5>{});
+      default: break;
+    }
+  } else if (in == b200collFloat8e4m3) {
+    switch (out) {
+      case b200collFloat8e4m3: return f(Tag<f8>{}, Tag<f8>{});
+      case b200collBfloat16: return f(Tag<f8>{}, Tag<bf16>{});
+      case b200collFloat16: return f(Tag<f8>{}, Tag<__half>{});
+      case b200collFloat32: return f(Tag<f8>{}, Tag<float>{});
+      default: break;
+    }
+  } else if (in == b200collFloat8e5m2) {
+    switch (out) {
+      case b200collFloat8e5m2: return f(Tag<f8e5>{}, Tag<f8e5>{});
+      case b200collBfloat16: return f(Tag<f8e5>{}, Tag<bf16>{});
+      case b200collFloat16: return f(Tag<f8e5>{}, Tag<__half>{});
+      case b200collFloat32: return f(Tag<f8e5>{}, Tag<float>{});
       default: break;
     }
   }
   set_last_error("unsupported (in_dtype, out_dtype) pair");
   return b200collInvalidArgument;
 }
+
+// No multicast (NVLS) kernel is built for an fp8 input: the switch reduces fp8 with an f16 accumulator only (ptxas refuses .acc::f32
+// for e4m3x4 / e5m2x4), and those kernels have not yet run on a multi-GPU NVSwitch system. An fp8 call the tuner sends to NVLS takes
+// two-shot, and the Lamport kernels write their slots with P2P stores instead of multimem.st. `if constexpr` keeps the fp8 multicast
+// instantiations out of the library altogether.
+template <typename T> constexpr bool kMcKernels = !IsFp8<T>::value;
+static bool is_fp8(b200collDataType_t t) { return t == b200collFloat8e4m3 || t == b200collFloat8e5m2; }
 
 #define LAUNCH_CHECK(c)                                                                                  \
   do {                                                                                                   \
@@ -129,7 +157,8 @@ static size_t out_align(size_t in_sz, size_t out_sz) { return std::min<size_t>(1
 
 static b200collResult_t check_common(b200collComm* c, const void* send, void* recv, const b200collEpilogue* ep) {
   if (!c || !send || !recv || !ep) { set_last_error("null argument"); return b200collInvalidArgument; }
-  if ((int)ep->in_dtype < 0 || (int)ep->in_dtype >= (int)b200collFloat8e4m3 || (int)ep->out_dtype < 0 || (int)ep->out_dtype > (int)b200collFloat8e4m3) { set_last_error("bad dtype (fp32 / fp16 / bf16 in, those or e4m3 out; integer and fp64 payloads: reductions take the generic path, data movement takes them as words)"); return b200collInvalidArgument; }
+  auto fused = [](b200collDataType_t t) { return ((int)t >= 0 && (int)t <= (int)b200collFloat8e4m3) || t == b200collFloat8e5m2; };
+  if (!fused(ep->in_dtype) || !fused(ep->out_dtype)) { set_last_error("bad dtype (fp32 / fp16 / bf16 / fp8 e4m3 / fp8 e5m2 in and out; integer and fp64 payloads: reductions take the generic path, data movement takes them as words)"); return b200collInvalidArgument; }
   const size_t is = b200collTypeSize(ep->in_dtype), os = b200collTypeSize(ep->out_dtype);
   if (!aligned(send, 16) || !aligned(recv, out_align(is, os))) { set_last_error("send must be 16-byte aligned and recv aligned to one output vector"); return b200collInvalidArgument; }
   if (c->fault_host && *const_cast<volatile uint32_t*>(&c->fault_host->code) != 0) { set_last_error("communicator is poisoned by an earlier watchdog fault"); return b200collRemoteError; }
@@ -244,15 +273,15 @@ static b200collResult_t launch_ll(b200collComm* c, b200collOp_t op, const void* 
     const size_t nv = (count + E - 1) / E;
     Grid g = pick_grid(c, kShapeLL, nv, 1);
     const InT* in = static_cast<const InT*>(send); OutT* out = static_cast<OutT*>(recv);
-    const bool mc = c->nvls;
+    const bool mc = c->nvls && kMcKernels<InT>;
     struct PdlScope { PdlScope(bool v) { t_pdl_small = v; } ~PdlScope() { t_pdl_small = false; } } pdl_scope(count * sizeof(InT) <= pdl_max_bytes());
     switch (op) {
       case b200collOpAllReduce:
-        if (mc) launch_k(k_ll<InT, OutT, false, true, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
+        if (mc) { if constexpr (kMcKernels<InT>) launch_k(k_ll<InT, OutT, false, true, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); }
         else launch_k(k_ll<InT, OutT, false, true, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
         break;
       case b200collOpAllGather:
-        if (mc) launch_k(k_ll<InT, OutT, false, false, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
+        if (mc) { if constexpr (kMcKernels<InT>) launch_k(k_ll<InT, OutT, false, false, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); }
         else launch_k(k_ll<InT, OutT, false, false, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
         break;
       case b200collOpReduceScatter:
@@ -273,7 +302,7 @@ static b200collResult_t launch_ll2_typed(b200collComm* c, const void* send, void
   constexpr int E = Epv<InT>::value;
   const size_t nslice = ((count + E - 1) / E + c->nranks - 1) / c->nranks;
   Grid g = pick_grid(c, kShapeLL, nslice, 1);
-  if (c->nvls) launch_k(k_ll_twoshot<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce);
+  if (c->nvls && kMcKernels<InT>) { if constexpr (kMcKernels<InT>) launch_k(k_ll_twoshot<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce); }
   else launch_k(k_ll_twoshot<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce);
   LAUNCH_CHECK(c);
   return b200collSuccess;
@@ -283,6 +312,8 @@ static b200collResult_t launch_ll2(b200collComm* c, const void* send, void* recv
   if (i == b200collFloat32 && o == b200collFloat32) return launch_ll2_typed<float, float>(c, send, recv, count, scale, st);
   if (i == b200collBfloat16 && o == b200collBfloat16) return launch_ll2_typed<bf16, bf16>(c, send, recv, count, scale, st);
   if (i == b200collFloat16 && o == b200collFloat16) return launch_ll2_typed<__half, __half>(c, send, recv, count, scale, st);
+  if (i == b200collFloat8e4m3 && o == b200collFloat8e4m3) return launch_ll2_typed<f8, f8>(c, send, recv, count, scale, st);
+  if (i == b200collFloat8e5m2 && o == b200collFloat8e5m2) return launch_ll2_typed<f8e5, f8e5>(c, send, recv, count, scale, st);
   set_last_error("two-shot LL needs in_dtype == out_dtype");
   return b200collInvalidArgument;
 }
@@ -301,6 +332,9 @@ static b200collResult_t ar_symmetric(b200collComm* c, b200collAlgo_t algo, const
     } else if (algo == b200collAlgoTwoShot) {
       Grid g = pick_grid(c, kShapeP2p, nvec / c->nranks + 1, 2);
       launch_k(k_ar_twoshot<InT, OutT>, g.blocks, g.threads, st, c->dev, in_off, arena_off(c, recv), count, scale, b200collOpAllReduce);
+    } else if constexpr (!kMcKernels<InT>) {
+      set_last_error("no NVLS all-reduce kernel for fp8 inputs");
+      return b200collInternalError;
     } else {
       static const int forced_u = [] { const char* e = getenv("B200COLL_NVLS_UNROLL"); return e ? atoi(e) : 0; }();
       const size_t slice = nvec / c->nranks + 1;
@@ -492,7 +526,7 @@ b200collResult_t b200collAllReduce(const void* send, void* recv, size_t count, c
       case b200collAlgoLL2: return is == os && bytes <= kLLOneShotMaxBytes * (size_t)c->nranks;
       case b200collAlgoOneShot: return sym_in && !inplace;
       case b200collAlgoTwoShot: return sym_in && sym_out;
-      case b200collAlgoNvls: return c->nvls && sym_in && sym_out;
+      case b200collAlgoNvls: return c->nvls && sym_in && sym_out && !is_fp8(ep->in_dtype);   // see kMcKernels
       default: return false;
     }
   };
@@ -511,7 +545,7 @@ b200collResult_t b200collAllReduce(const void* send, void* recv, size_t count, c
   }
   // ---- staged: buffers outside the arena and too big for LL. Chunk through the two staging halves.
   c->stats.staged_calls++;
-  b200collAlgo_t inner = (c->nvls && c->nranks > 2) ? b200collAlgoNvls : b200collAlgoTwoShot;
+  b200collAlgo_t inner = (c->nvls && c->nranks > 2 && !is_fp8(ep->in_dtype)) ? b200collAlgoNvls : b200collAlgoTwoShot;
   const size_t chunk = std::min(kStageHalfBytes / is, kStageHalfBytes / os) / 64 * 64;
   for (size_t done = 0; done < count; done += chunk) {
     const size_t n = std::min(chunk, count - done);
@@ -541,7 +575,7 @@ b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcoun
   if (algo == b200collAlgoOneShot) algo = b200collAlgoTwoShot;
   if (algo == b200collAlgoLL2) algo = b200collAlgoLL;
   if (algo == b200collAlgoLL && bytes > kLLOneShotMaxBytes) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoNvls && !c->nvls) algo = b200collAlgoTwoShot;
+  if (algo == b200collAlgoNvls && (!c->nvls || is_fp8(ep->in_dtype))) algo = b200collAlgoTwoShot;   // fp8: see kMcKernels
   if (algo == b200collAlgoLL) { account(c, b200collOpAllGather, bytes, algo); return launch_ll(c, b200collOpAllGather, send, recv, sendcount, ep, scale, st); }
   const int identity = (ep->in_dtype == ep->out_dtype && scale == 1.0f) ? 1 : 0;
   auto push = [&](const void* s, void* r, size_t n) -> b200collResult_t {
@@ -549,7 +583,7 @@ b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcoun
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeNvls : kShapeP2p, n / Epv<InT>::value, 4);
-      if (algo == b200collAlgoNvls) launch_k(k_ag_push<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather);
+      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_ag_push<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather); }
       else launch_k(k_ag_push<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather);
       LAUNCH_CHECK(c);
       return b200collSuccess;
@@ -599,14 +633,14 @@ b200collResult_t b200collReduceScatter(const void* send, void* recv, size_t recv
   if (algo == b200collAlgoOneShot) algo = b200collAlgoTwoShot;
   if (algo == b200collAlgoLL2) algo = b200collAlgoLL;
   if (algo == b200collAlgoLL && bytes > kLLOneShotMaxBytes) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoNvls && !c->nvls) algo = b200collAlgoTwoShot;
+  if (algo == b200collAlgoNvls && (!c->nvls || is_fp8(ep->in_dtype))) algo = b200collAlgoTwoShot;   // fp8: see kMcKernels
   if (algo == b200collAlgoLL) { account(c, b200collOpReduceScatter, bytes, algo); return launch_ll(c, b200collOpReduceScatter, send, recv, recvcount, ep, scale, st); }
   auto pull = [&](const void* s_slice_of_mine, void* r, size_t n) -> b200collResult_t {
     account(c, b200collOpReduceScatter, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeNvlsRs : kShapeP2p, n / Epv<InT>::value, 2);
-      if (algo == b200collAlgoNvls) launch_k(k_pull_reduce<InT, OutT, false, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter);
+      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_pull_reduce<InT, OutT, false, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter); }
       else launch_k(k_pull_reduce<InT, OutT, false, false>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter);
       LAUNCH_CHECK(c);
       return b200collSuccess;
@@ -757,14 +791,14 @@ b200collResult_t b200collBroadcast(const void* send, void* recv, size_t count, c
   if (c->nranks == 1) { account(c, b200collOpBroadcast, count * is, b200collAlgoCopy); return copy_scale(c, send, recv, count, ep, scale, st); }
   if (send == recv && is != os) { set_last_error("in-place broadcast needs in_dtype and out_dtype of equal size"); return b200collInvalidArgument; }
   b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpBroadcast, count * is, c->nranks, c->nvls);
-  if (algo != b200collAlgoNvls || !c->nvls) algo = b200collAlgoTwoShot;     // two families only: multimem.st or P2P push
+  if (algo != b200collAlgoNvls || !c->nvls || is_fp8(ep->in_dtype)) algo = b200collAlgoTwoShot;     // two families only: multimem.st or P2P push
   const int identity = (ep->in_dtype == ep->out_dtype && scale == 1.0f) ? 1 : 0;
   auto push = [&](const void* s, void* r_sym, size_t n) -> b200collResult_t {
     account(c, b200collOpBroadcast, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeRooted : kShapeP2p, std::max<size_t>(1, n / Epv<InT>::value), 4);
-      if (algo == b200collAlgoNvls) launch_k(k_bcast<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast);
+      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_bcast<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast); }
       else launch_k(k_bcast<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast);
       LAUNCH_CHECK(c);
       return b200collSuccess;
@@ -808,13 +842,13 @@ b200collResult_t b200collReduce(const void* send, void* recv, size_t count, cons
   if (c->nranks == 1) { account(c, b200collOpReduce, count * is, b200collAlgoCopy); return copy_scale(c, send, recv, count, ep, scale, st); }
   if (send == recv && is != os) { set_last_error("in-place reduce needs in_dtype and out_dtype of equal size"); return b200collInvalidArgument; }
   b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpReduce, count * is, c->nranks, c->nvls);
-  if (algo != b200collAlgoNvls || !c->nvls) algo = b200collAlgoTwoShot;     // multimem.ld_reduce by the root, or the root pulls from every peer
+  if (algo != b200collAlgoNvls || !c->nvls || is_fp8(ep->in_dtype)) algo = b200collAlgoTwoShot;     // multimem.ld_reduce by the root, or the root pulls from every peer
   auto pull = [&](const void* s_sym, void* r, size_t n) -> b200collResult_t {
     account(c, b200collOpReduce, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeRooted : kShapeP2p, std::max<size_t>(1, n / Epv<InT>::value), algo == b200collAlgoNvls ? 4 : 2);
-      if (algo == b200collAlgoNvls) launch_k(k_reduce_root<InT, OutT, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce);
+      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_reduce_root<InT, OutT, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce); }
       else launch_k(k_reduce_root<InT, OutT, false>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce);
       LAUNCH_CHECK(c);
       return b200collSuccess;

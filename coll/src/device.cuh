@@ -3,7 +3,7 @@
 //   * epoch barrier over per-block flags in each rank's control page (monotonic, never reset)
 //   * Lamport (flag-in-payload) slot protocol for the zero-barrier small-message path
 //   * multimem.{ld_reduce,st} wrappers (NVLS: reduce / broadcast inside the NVSwitch)
-//   * 16-byte vector load/convert/store for {f32,f16,bf16} in and {f32,f16,bf16,e4m3} out
+//   * 16-byte vector load/convert/store for {f32,f16,bf16,e4m3,e5m2} in and out (fp8: 16 elements per vector)
 // Every cross-GPU spin carries a globaltimer watchdog that records a b200collFault and bails
 // out instead of hanging the GPU (SURVEY §5.3).
 #pragma once
@@ -174,6 +174,27 @@ template <> __device__ __forceinline__ void unpack_add<__half>(float* acc, const
     acc[2 * i] += f.x; acc[2 * i + 1] += f.y;
   }
 }
+// fp8: 16 elements per vector. fp8 -> f16 -> f32 is exact for both encodings (every e4m3 / e5m2 value is an f16 value); the low byte
+// of each word is the lower-indexed element, as Pack<fp8> writes it.
+template <__nv_fp8_interpretation_t K>
+__device__ __forceinline__ void unpack_add_fp8(float* acc, const uint4& v) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+  for (int i = 0; i < 4; i++) {
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+      const __half2 p = __half2(__nv_cvt_fp8x2_to_halfraw2((__nv_fp8x2_storage_t)(w[i] >> (16 * h)), K));
+      const float2 f = __half22float2(p);
+      acc[4 * i + 2 * h] += f.x; acc[4 * i + 2 * h + 1] += f.y;
+    }
+  }
+}
+template <> __device__ __forceinline__ void unpack_add<__nv_fp8_e4m3>(float* acc, const uint4& v) { unpack_add_fp8<__NV_E4M3>(acc, v); }
+template <> __device__ __forceinline__ void unpack_add<__nv_fp8_e5m2>(float* acc, const uint4& v) { unpack_add_fp8<__NV_E5M2>(acc, v); }
+
+template <typename T> struct IsFp8 { static constexpr bool value = false; };
+template <> struct IsFp8<__nv_fp8_e4m3> { static constexpr bool value = true; };
+template <> struct IsFp8<__nv_fp8_e5m2> { static constexpr bool value = true; };
 
 // pack E floats into E*sizeof(OutT)/4 words
 template <typename OutT, int E> struct Pack;
@@ -209,8 +230,24 @@ template <int E> struct Pack<__nv_fp8_e4m3, E> {
     }
   }
 };
+template <int E> struct Pack<__nv_fp8_e5m2, E> {
+  static constexpr int W = E / 4;
+  static __device__ __forceinline__ void run(const float* f, uint32_t* w) {
+#pragma unroll
+    for (int i = 0; i < E / 4; i++) {
+      uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(f[4 * i], f[4 * i + 1]), __NV_SATFINITE, __NV_E5M2);
+      uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(f[4 * i + 2], f[4 * i + 3]), __NV_SATFINITE, __NV_E5M2);
+      w[i] = lo | (hi << 16);
+    }
+  }
+};
 
 template <int W> __device__ __forceinline__ void st_words(void* p, const uint32_t* w) {
+  if constexpr (W == 16) {   // fp8 in, fp32 out: one input vector widens to 64 bytes
+#pragma unroll
+    for (int q = 0; q < 4; q++) st_vec(reinterpret_cast<char*>(p) + 16 * q, make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]));
+    return;
+  }
   if (W == 8) {
     st_vec(p, make_uint4(w[0], w[1], w[2], w[3]));
     st_vec(reinterpret_cast<char*>(p) + 16, make_uint4(w[4], w[5], w[6], w[7]));
@@ -235,6 +272,19 @@ template <typename T> __device__ __forceinline__ T from_float(float v);
 template <> __device__ __forceinline__ float from_float<float>(float v) { return v; }
 template <> __device__ __forceinline__ __half from_float<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 from_float<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-template <> __device__ __forceinline__ __nv_fp8_e4m3 from_float<__nv_fp8_e4m3>(float v) { return __nv_fp8_e4m3(v); }
+template <> __device__ __forceinline__ __nv_fp8_e4m3 from_float<__nv_fp8_e4m3>(float v) { return __nv_fp8_e4m3(v); }   // round to nearest, saturate to +-448
+template <> __device__ __forceinline__ __nv_fp8_e5m2 from_float<__nv_fp8_e5m2>(float v) { return __nv_fp8_e5m2(v); }   // round to nearest, saturate to +-57344
+template <> __device__ __forceinline__ float to_float<__nv_fp8_e4m3>(__nv_fp8_e4m3 v) { return float(v); }
+template <> __device__ __forceinline__ float to_float<__nv_fp8_e5m2>(__nv_fp8_e5m2 v) { return float(v); }
+
+// Element e of a peer's buffer, read with a volatile load (scalar tails). The fp8 classes cannot be copied from a volatile object,
+// so their byte is loaded as a plain integer and reinterpreted.
+template <typename T> __device__ __forceinline__ float ld_volatile_float(const char* base, size_t e) { return to_float<T>(reinterpret_cast<const volatile T*>(base)[e]); }
+template <> __device__ __forceinline__ float ld_volatile_float<__nv_fp8_e4m3>(const char* base, size_t e) {
+  __nv_fp8_e4m3 v; v.__x = reinterpret_cast<const volatile __nv_fp8_storage_t*>(base)[e]; return float(v);
+}
+template <> __device__ __forceinline__ float ld_volatile_float<__nv_fp8_e5m2>(const char* base, size_t e) {
+  __nv_fp8_e5m2 v; v.__x = reinterpret_cast<const volatile __nv_fp8_storage_t*>(base)[e]; return float(v);
+}
 
 }  // namespace b200coll

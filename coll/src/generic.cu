@@ -3,7 +3,7 @@
 // int64 all-reduces, nccl-tests `-o max -d int32`, a MIN over step counters (reference role: the installed NCCL,
 // gpudirect-tcpxo/README.md:66-70, takes all of ncclRedOp_t x ncclDataType_t).
 // One barrier-based P2P kernel (no Lamport path: its empty-slot marker is a NaN pattern, which is a legal integer; no NVLS: the
-// switch has no prod and no 64-bit integer min/max), accumulating in the element type (fp16 / bf16 in fp32), in rank order, so every
+// switch has no prod and no 64-bit integer min/max), accumulating in the element type (fp16 / bf16 / fp8 in fp32), in rank order, so every
 // rank computes bit-identical results:
 //   all-reduce      rank r pulls vector slice r from every peer, reduces, pushes the result into every peer's out   (two-shot)
 //   reduce-scatter  rank r pulls its block from every peer, reduces into its local out
@@ -22,12 +22,22 @@ enum { kModeAllReduce = 0, kModeToLocal = 1 };
 template <typename T> struct GAcc { using type = T; };
 template <> struct GAcc<__half> { using type = float; };
 template <> struct GAcc<__nv_bfloat16> { using type = float; };
+template <> struct GAcc<__nv_fp8_e4m3> { using type = float; };
+template <> struct GAcc<__nv_fp8_e5m2> { using type = float; };
 template <typename T> __device__ __forceinline__ typename GAcc<T>::type g_load(T v) { return (typename GAcc<T>::type)v; }
 template <> __device__ __forceinline__ float g_load<__half>(__half v) { return __half2float(v); }
 template <> __device__ __forceinline__ float g_load<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <> __device__ __forceinline__ float g_load<__nv_fp8_e4m3>(__nv_fp8_e4m3 v) { return float(v); }
+template <> __device__ __forceinline__ float g_load<__nv_fp8_e5m2>(__nv_fp8_e5m2 v) { return float(v); }
 template <typename T> __device__ __forceinline__ T g_store(typename GAcc<T>::type v) { return (T)v; }
 template <> __device__ __forceinline__ __half g_store<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 g_store<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __nv_fp8_e4m3 g_store<__nv_fp8_e4m3>(float v) { return __nv_fp8_e4m3(v); }   // saturating, like the fused paths
+template <> __device__ __forceinline__ __nv_fp8_e5m2 g_store<__nv_fp8_e5m2>(float v) { return __nv_fp8_e5m2(v); }
+// scalar tails read peers' elements with volatile loads; the fp8 classes cannot be copied from a volatile object
+template <typename T> __device__ __forceinline__ typename GAcc<T>::type g_load_volatile(const char* base, size_t e) { return g_load<T>(reinterpret_cast<const volatile T*>(base)[e]); }
+template <> __device__ __forceinline__ float g_load_volatile<__nv_fp8_e4m3>(const char* base, size_t e) { return ld_volatile_float<__nv_fp8_e4m3>(base, e); }
+template <> __device__ __forceinline__ float g_load_volatile<__nv_fp8_e5m2>(const char* base, size_t e) { return ld_volatile_float<__nv_fp8_e5m2>(base, e); }
 
 template <int OP, typename A> __device__ __forceinline__ A g_apply(A a, A b) {
   if (OP == b200collSum) return a + b;
@@ -91,8 +101,8 @@ __global__ void __launch_bounds__(512) k_generic_reduce(COMM_PARAM, size_t in_of
     if (blockIdx.x == 0 && (mode != kModeAllReduce || c.rank == 0)) {
       const size_t e = nvec * E + threadIdx.x;
       if (e < count) {
-        A acc = g_load<T>(reinterpret_cast<const volatile T*>(c.peer[0] + in_off)[e]);
-        for (int r = 1; r < c.nranks; r++) acc = g_apply<OP, A>(acc, g_load<T>(reinterpret_cast<const volatile T*>(c.peer[r] + in_off)[e]));
+        A acc = g_load_volatile<T>(c.peer[0] + in_off, e);
+        for (int r = 1; r < c.nranks; r++) acc = g_apply<OP, A>(acc, g_load_volatile<T>(c.peer[r] + in_off, e));
         const T o = g_store<T>(acc);
         if (mode == kModeAllReduce) { for (int r = 0; r < c.nranks; r++) reinterpret_cast<T*>(c.peer[r] + out_off)[e] = o; }
         else out_local[e] = o;
@@ -137,12 +147,15 @@ static b200collResult_t dispatch_generic(b200collComm* c, b200collDataType_t dt,
     case b200collFloat32: return launch_generic<float>(c, rop, in_off, out_off, out_local, count, mode, worker, op, st);
     case b200collFloat16: return launch_generic<__half>(c, rop, in_off, out_off, out_local, count, mode, worker, op, st);
     case b200collBfloat16: return launch_generic<__nv_bfloat16>(c, rop, in_off, out_off, out_local, count, mode, worker, op, st);
+    case b200collFloat8e4m3: return launch_generic<__nv_fp8_e4m3>(c, rop, in_off, out_off, out_local, count, mode, worker, op, st);
+    case b200collFloat8e5m2: return launch_generic<__nv_fp8_e5m2>(c, rop, in_off, out_off, out_local, count, mode, worker, op, st);
     default: set_last_error("unsupported dtype for a generic reduction"); return b200collInvalidArgument;
   }
 }
 
 bool needs_generic(const b200collEpilogue* ep, b200collRedOp_t rop) {
-  const bool fp = ep->in_dtype == b200collFloat32 || ep->in_dtype == b200collFloat16 || ep->in_dtype == b200collBfloat16;
+  const bool fp = ep->in_dtype == b200collFloat32 || ep->in_dtype == b200collFloat16 || ep->in_dtype == b200collBfloat16 ||
+                  ep->in_dtype == b200collFloat8e4m3 || ep->in_dtype == b200collFloat8e5m2;
   return !fp || rop == b200collProd || rop == b200collMin || rop == b200collMax;
 }
 
@@ -150,9 +163,9 @@ bool needs_generic(const b200collEpilogue* ep, b200collRedOp_t rop) {
 // b200collOpReduce (count = elements, root). One rank: a copy. Non-symmetric buffers: chunked through the staging halves.
 b200collResult_t generic_reduce(b200collComm* c, b200collOp_t which, const void* send, void* recv, size_t count, const b200collEpilogue* ep, b200collRedOp_t rop, int root, cudaStream_t st) {
   if (ep->in_dtype != ep->out_dtype || ep->scale != 1.0f) { set_last_error("min / max / prod and integer / fp64 reductions take no cast or scale (in_dtype == out_dtype, scale == 1)"); return b200collInvalidArgument; }
-  if (rop == b200collAvg) { set_last_error("avg is defined for fp16 / bf16 / fp32 only"); return b200collInvalidArgument; }
+  if (rop == b200collAvg) { set_last_error("avg is defined for fp32 / fp16 / bf16 / fp8 only"); return b200collInvalidArgument; }
   const size_t es = b200collTypeSize(ep->in_dtype);
-  if (es == 0 || ep->in_dtype == b200collFloat8e4m3) { set_last_error("bad dtype"); return b200collInvalidArgument; }
+  if (es == 0) { set_last_error("bad dtype"); return b200collInvalidArgument; }
   if (reinterpret_cast<uintptr_t>(send) % 16 || reinterpret_cast<uintptr_t>(recv) % 16) { set_last_error("send and recv must be 16-byte aligned"); return b200collInvalidArgument; }
   if (c->fault_host && *const_cast<volatile uint32_t*>(&c->fault_host->code) != 0) { set_last_error("communicator is poisoned by an earlier watchdog fault"); return b200collRemoteError; }
   if (count == 0) return b200collSuccess;

@@ -288,7 +288,7 @@ __device__ __forceinline__ void ar_tail_rank0(const CommDev& c, size_t in_off, s
   const size_t e = e0 + threadIdx.x;
   if (e >= count) return;
   float acc = 0.f;
-  for (int r = 0; r < c.nranks; r++) acc += to_float<InT>(reinterpret_cast<const volatile InT*>(c.peer[r] + in_off)[e]);
+  for (int r = 0; r < c.nranks; r++) acc += ld_volatile_float<InT>(c.peer[r] + in_off, e);
   const OutT o = from_float<OutT>(acc * scale);
   for (int r = 0; r < c.nranks; r++) reinterpret_cast<OutT*>(c.peer[r] + out_off)[e] = o;
 }
@@ -305,7 +305,7 @@ __global__ void __launch_bounds__(kThreads) k_pull_reduce(COMM_PARAM, size_t in_
   const size_t nvec = count / E;
   const size_t stride = (size_t)gridDim.x * blockDim.x * U;
   for (size_t base = (size_t)blockIdx.x * blockDim.x * U + threadIdx.x; base < nvec; base += stride) {
-    if (MC) {
+    if constexpr (MC) {   // constexpr: the non-MC instantiation must not reference mc_ld_reduce<InT> (none exists for fp8)
       uint4 d[U];
 #pragma unroll
       for (int u = 0; u < U; u++) { const size_t v = base + (size_t)u * blockDim.x; if (v < nvec) d[u] = mc_ld_reduce<InT>(c.mc + in_off + v * 16); }
@@ -344,7 +344,7 @@ __global__ void __launch_bounds__(kThreads) k_pull_reduce(COMM_PARAM, size_t in_
     const size_t e = nvec * E + threadIdx.x;
     if (e < count) {
       float acc = 0.f;
-      for (int r = 0; r < c.nranks; r++) acc += to_float<InT>(reinterpret_cast<const volatile InT*>(c.peer[r] + in_off)[e]);
+      for (int r = 0; r < c.nranks; r++) acc += ld_volatile_float<InT>(c.peer[r] + in_off, e);
       out[e] = from_float<OutT>(acc * scale);
     }
   }
@@ -637,7 +637,7 @@ __global__ void __launch_bounds__(kThreads) k_reduce_root(COMM_PARAM, size_t in_
     const size_t nvec = count / E;
     const size_t stride = (size_t)gridDim.x * blockDim.x * U;
     for (size_t base = (size_t)blockIdx.x * blockDim.x * U + threadIdx.x; base < nvec; base += stride) {
-      if (MC) {
+      if constexpr (MC) {
         uint4 d[U];
 #pragma unroll
         for (int u = 0; u < U; u++) { const size_t v = base + (size_t)u * blockDim.x; if (v < nvec) d[u] = mc_ld_reduce<InT>(c.mc + in_off + v * 16); }
@@ -672,7 +672,7 @@ __global__ void __launch_bounds__(kThreads) k_reduce_root(COMM_PARAM, size_t in_
       const size_t e = nvec * E + threadIdx.x;
       if (e < count) {
         float acc = 0.f;
-        for (int r = 0; r < c.nranks; r++) acc += to_float<InT>(reinterpret_cast<const volatile InT*>(c.peer[r] + in_off)[e]);
+        for (int r = 0; r < c.nranks; r++) acc += ld_volatile_float<InT>(c.peer[r] + in_off, e);
         out[e] = from_float<OutT>(acc * scale);
       }
     }

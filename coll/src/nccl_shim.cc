@@ -20,7 +20,8 @@ extern "C" {
 typedef struct ncclComm* ncclComm_t;
 typedef struct { char internal[128]; } ncclUniqueId;
 typedef enum { ncclSuccess = 0, ncclUnhandledCudaError = 1, ncclSystemError = 2, ncclInternalError = 3, ncclInvalidArgument = 4, ncclInvalidUsage = 5, ncclRemoteError = 6, ncclInProgress = 7 } ncclResult_t;
-typedef enum { ncclInt8 = 0, ncclUint8 = 1, ncclInt32 = 2, ncclUint32 = 3, ncclInt64 = 4, ncclUint64 = 5, ncclFloat16 = 6, ncclFloat32 = 7, ncclFloat64 = 8, ncclBfloat16 = 9 } ncclDataType_t;
+typedef enum { ncclInt8 = 0, ncclUint8 = 1, ncclInt32 = 2, ncclUint32 = 3, ncclInt64 = 4, ncclUint64 = 5, ncclFloat16 = 6, ncclFloat32 = 7, ncclFloat64 = 8, ncclBfloat16 = 9,
+               ncclFloat8e4m3 = 10, ncclFloat8e5m2 = 11, ncclNumTypes = 12 } ncclDataType_t;
 typedef enum { ncclSum = 0, ncclProd = 1, ncclMax = 2, ncclMin = 3, ncclAvg = 4 } ncclRedOp_t;
 typedef enum { ncclScalarDevice = 0, ncclScalarHostImmediate = 1 } ncclScalarResidence_t;
 typedef struct ncclWindow_vidmem* ncclWindow_t;
@@ -55,11 +56,12 @@ bool map_dt(ncclDataType_t dt, b200collDataType_t* out) {
     case ncclFloat32: *out = b200collFloat32; return true;
     case ncclFloat16: *out = b200collFloat16; return true;
     case ncclBfloat16: *out = b200collBfloat16; return true;
-    default: return false;   // integer / fp64: reductions go through map_dt_reduce (generic kernel), data movement through map_dt_as_words
+    default: return false;   // integer / fp64 / fp8: reductions go through map_dt_reduce, data movement through map_dt_as_words
   }
 }
 
-// Every NCCL element type that libb200coll can reduce (fp8 is a wire / output format only, as in NCCL before 2.24).
+// Every NCCL element type that libb200coll can reduce, fp8 included (NCCL reduces e4m3 / e5m2 since 2.24): fp8 sum / avg / PreMulSum
+// run on the fused fp32-accumulating kernels, min / max / prod and the integer / fp64 types on the generic kernel.
 bool map_dt_reduce(ncclDataType_t dt, b200collDataType_t* out) {
   switch (dt) {
     case ncclInt8: *out = b200collInt8; return true;
@@ -69,6 +71,8 @@ bool map_dt_reduce(ncclDataType_t dt, b200collDataType_t* out) {
     case ncclInt64: *out = b200collInt64; return true;
     case ncclUint64: *out = b200collUint64; return true;
     case ncclFloat64: *out = b200collFloat64; return true;
+    case ncclFloat8e4m3: *out = b200collFloat8e4m3; return true;
+    case ncclFloat8e5m2: *out = b200collFloat8e5m2; return true;
     default: return map_dt(dt, out);
   }
 }
@@ -93,7 +97,7 @@ bool map_op(ncclRedOp_t op, b200collRedOp_t* rop, float* scale) {
 
 size_t nccl_type_size(ncclDataType_t dt) {
   switch ((int)dt) {
-    case ncclInt8: case ncclUint8: case 10 /* ncclFloat8e4m3 */: case 11 /* ncclFloat8e5m2 */: return 1;
+    case ncclInt8: case ncclUint8: case ncclFloat8e4m3: case ncclFloat8e5m2: return 1;
     case ncclFloat16: case ncclBfloat16: return 2;
     case ncclInt32: case ncclUint32: case ncclFloat32: return 4;
     case ncclInt64: case ncclUint64: case ncclFloat64: return 8;
@@ -299,10 +303,11 @@ ncclResult_t ncclReduceScatter(const void* send, void* recv, size_t recvcount, n
 }
 
 // Broadcast moves bits, so every NCCL dtype works: the payload is described to the library as f16/f32 words
-// (scale 1, same type in and out = the bit-exact identity path).
+// (scale 1, same type in and out = the bit-exact identity path). fp8 goes this way too, not through the typed fp8 kernels: NCCL's
+// movement ops are bit-exact, and the Lamport path would rewrite a payload word that equals its empty-slot marker.
 static bool map_dt_as_words(ncclDataType_t dt, size_t count, b200collDataType_t* t, size_t* n) {
   switch (dt) {
-    case ncclInt8: case ncclUint8: if (count % 2) return false; *t = b200collFloat16; *n = count / 2; return true;
+    case ncclInt8: case ncclUint8: case ncclFloat8e4m3: case ncclFloat8e5m2: if (count % 2) return false; *t = b200collFloat16; *n = count / 2; return true;
     case ncclFloat16: case ncclBfloat16: *t = b200collFloat16; *n = count; return true;
     case ncclInt32: case ncclUint32: case ncclFloat32: *t = b200collFloat32; *n = count; return true;
     case ncclInt64: case ncclUint64: case ncclFloat64: *t = b200collFloat32; *n = count * 2; return true;

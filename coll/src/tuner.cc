@@ -120,7 +120,7 @@ size_t b200collTypeSize(b200collDataType_t t) {
     case b200collFloat32: return 4;
     case b200collFloat16: return 2;
     case b200collBfloat16: return 2;
-    case b200collFloat8e4m3: return 1;
+    case b200collFloat8e4m3: case b200collFloat8e5m2: return 1;
     case b200collInt8: case b200collUint8: return 1;
     case b200collInt32: case b200collUint32: return 4;
     case b200collInt64: case b200collUint64: case b200collFloat64: return 8;

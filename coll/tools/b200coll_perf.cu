@@ -63,11 +63,13 @@ static b200collDataType_t parse_dt(const char* s) {
   if (!strcmp(s, "f16") || !strcmp(s, "half")) return b200collFloat16;
   if (!strcmp(s, "bf16") || !strcmp(s, "bfloat16")) return b200collBfloat16;
   if (!strcmp(s, "fp8") || !strcmp(s, "e4m3")) return b200collFloat8e4m3;
+  if (!strcmp(s, "e5m2")) return b200collFloat8e5m2;
   fprintf(stderr, "bad dtype %s\n", s); exit(1);
 }
-static const char* dt_name(b200collDataType_t t) { return t == b200collFloat32 ? "f32" : t == b200collFloat16 ? "f16" : t == b200collBfloat16 ? "bf16" : "e4m3"; }
+static const char* dt_name(b200collDataType_t t) { return t == b200collFloat32 ? "f32" : t == b200collFloat16 ? "f16" : t == b200collBfloat16 ? "bf16" : t == b200collFloat8e5m2 ? "e5m2" : "e4m3"; }
 
-// deterministic input: multiples of 0.25 in [-2, 2] so sums over <= 8 ranks are exact in bf16/f16/f32
+// deterministic input: multiples of 0.25 in [-2, 2] so sums over <= 8 ranks are exact in bf16/f16/f32 (and in the fp32 accumulator
+// of the fp8 paths: every such value is an e4m3 and an e5m2 value)
 static inline float gen(int rank, size_t i) { return (float)((int)((i * 7 + (size_t)rank * 13 + (i >> 9)) % 17) - 8) * 0.25f; }
 
 template <typename T> __global__ void k_fill(T* p, size_t n, int rank, size_t base) {
@@ -80,6 +82,8 @@ template <typename T> __global__ void k_fill(T* p, size_t n, int rank, size_t ba
 static void fill(void* p, size_t n, b200collDataType_t dt, int rank, size_t base, cudaStream_t st) {
   if (dt == b200collFloat32) k_fill<float><<<256, 256, 0, st>>>((float*)p, n, rank, base);
   else if (dt == b200collFloat16) k_fill<__half><<<256, 256, 0, st>>>((__half*)p, n, rank, base);
+  else if (dt == b200collFloat8e4m3) k_fill<__nv_fp8_e4m3><<<256, 256, 0, st>>>((__nv_fp8_e4m3*)p, n, rank, base);
+  else if (dt == b200collFloat8e5m2) k_fill<__nv_fp8_e5m2><<<256, 256, 0, st>>>((__nv_fp8_e5m2*)p, n, rank, base);
   else k_fill<__nv_bfloat16><<<256, 256, 0, st>>>((__nv_bfloat16*)p, n, rank, base);
 }
 
@@ -88,8 +92,15 @@ static float to_f(const void* p, size_t i, b200collDataType_t dt) {
     case b200collFloat32: return ((const float*)p)[i];
     case b200collFloat16: return __half2float(((const __half*)p)[i]);
     case b200collBfloat16: return __bfloat162float(((const __nv_bfloat16*)p)[i]);
+    case b200collFloat8e5m2: return (float)(((const __nv_fp8_e5m2*)p)[i]);
     default: return (float)(((const __nv_fp8_e4m3*)p)[i]);
   }
+}
+// An exact fp32 result after the collective's saturating, round-to-nearest cast to `dt`.
+static float round_to(b200collDataType_t dt, float v) {
+  if (dt == b200collFloat8e4m3) return (float)__nv_fp8_e4m3(v);
+  if (dt == b200collFloat8e5m2) return (float)__nv_fp8_e5m2(v);
+  return v;
 }
 
 struct Shared {   // cross-process (mmap MAP_SHARED) or cross-thread rendezvous for timing
@@ -250,8 +261,12 @@ static int run_rank(const Opts& o, RankCtx ctx, Shared* sh) {
         RT(cudaMemcpy(host.data(), outp, check_elems * os, cudaMemcpyDeviceToHost));
         const size_t stride = check_elems > (1u << 22) ? 61 : 1;   // sample large buffers
         for (size_t e = 0; e < check_elems; e += stride) {
-          const float want = expected(o, rank, n, e, count), got = to_f(host.data(), e, o.out_dt);
-          const float tol = o.out_dt == b200collFloat8e4m3 ? fabsf(want) * 0.0725f + 0.002f : 0.0f;
+          // fp8 inputs accumulate exactly in fp32 (the fill's sums are exact), so the result is the exact sum rounded once: no tolerance
+          const bool fp8_in = o.in_dt == b200collFloat8e4m3 || o.in_dt == b200collFloat8e5m2;
+          float want = expected(o, rank, n, e, count);
+          if (fp8_in || o.out_dt == b200collFloat8e5m2) want = round_to(o.out_dt, want);
+          const float got = to_f(host.data(), e, o.out_dt);
+          const float tol = (!fp8_in && o.out_dt == b200collFloat8e4m3) ? fabsf(want) * 0.0725f + 0.002f : 0.0f;
           if (!(fabsf(got - want) <= tol)) { if (errs < 4) fprintf(stderr, "rank %d %s size %zu %s elem %zu: got %g want %g\n", rank, o.op.c_str(), bytes, ip ? "ip" : "oop", e, got, want); errs++; }
         }
       }
@@ -383,7 +398,7 @@ int main(int argc, char** argv) {
            "  -g N | --ranks N | --devs a,b,..   ranks in this process (threads); --procs forks one process per rank instead\n"
            "  under mpirun / torchrun (OMPI_COMM_WORLD_*, PMI_*, RANK/WORLD_SIZE/LOCAL_RANK) each process is one rank; B200COLL_JOB_ID names the job\n"
            "  -w N -n/--iters N -c 0|1  warm-up, timed iterations, check results against the host reference\n"
-           "  -d float|half|bfloat16    input type; --out-dtype T and --scale X fuse a cast / scale into the collective\n"
+           "  -d float|half|bfloat16|e4m3|e5m2   input type; --out-dtype T (same names) and --scale X fuse a cast / scale into the collective\n"
            "  --algo auto|ll|ll2|oneshot|twoshot|nvls   --inplace 0|1|2   --max-ctas N   --sweep kind:ctas:threads,...   --json FILE   --window SIZE\n"
            "  --selfcheck               report whether this node can run the NVLink fast paths (exit 1 if not)");
       return 0;

@@ -25,12 +25,12 @@ SUCCESS = 0
 NO_DRIVER = 9
 MAX_RANKS = 8
 
-F32, F16, BF16, FP8_E4M3, I8, U8, I32, U32, I64, U64, F64 = range(11)
+F32, F16, BF16, FP8_E4M3, I8, U8, I32, U32, I64, U64, F64, FP8_E5M2 = range(12)
 SUM, AVG, PROD, MIN, MAX = range(5)
 OP_ALLREDUCE, OP_ALLGATHER, OP_REDUCESCATTER, OP_ALLTOALL = 0, 1, 2, 3
 ALGO_AUTO, ALGO_LL, ALGO_ONESHOT, ALGO_TWOSHOT, ALGO_NVLS, ALGO_COPY, ALGO_LL2 = range(7)
 ALGO_NAMES = ["auto", "ll", "oneshot", "twoshot", "nvls", "copy", "ll2"]
-DTYPE_SIZE = {F32: 4, F16: 2, BF16: 2, FP8_E4M3: 1, I8: 1, U8: 1, I32: 4, U32: 4, I64: 8, U64: 8, F64: 8}
+DTYPE_SIZE = {F32: 4, F16: 2, BF16: 2, FP8_E4M3: 1, I8: 1, U8: 1, I32: 4, U32: 4, I64: 8, U64: 8, F64: 8, FP8_E5M2: 1}
 
 
 class UniqueId(C.Structure):
@@ -179,7 +179,7 @@ def self_check() -> tuple[bool, str]:
 
 def torch_dtype_code(dtype) -> int:
     import torch
-    return {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16, torch.float8_e4m3fn: FP8_E4M3, torch.int8: I8, torch.uint8: U8, torch.int32: I32,
+    return {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16, torch.float8_e4m3fn: FP8_E4M3, torch.float8_e5m2: FP8_E5M2, torch.int8: I8, torch.uint8: U8, torch.int32: I32,
             torch.int64: I64, torch.float64: F64, torch.bool: U8}[dtype]
 
 

@@ -6,7 +6,7 @@ of the NCCL API than nccl-tests does, so for PyTorch the faithful drop-in is a p
 
 How: a Python subclass of `torch.distributed.ProcessGroup` (c10d dispatches to it through its trampoline, the mechanism PyTorch's own
 tests use for Python process groups). CUDA tensors that the library can take as they are — contiguous, 16-byte aligned, fp32 / fp16 /
-bf16, sum or avg — go straight to the collective kernels **on the caller's current stream**, so ordering with the surrounding compute
+bf16 / fp8 (e4m3fn, e5m2), sum or avg — go straight to the collective kernels **on the caller's current stream**, so ordering with the surrounding compute
 is plain stream order and `Work.wait()` has nothing to wait for (NCCL's side stream + event dance is not needed). Tensors allocated
 with `pg.empty()` live in the symmetric arena and take the zero-copy / NVLS paths; any other device tensor is staged by the library.
 Point-to-point on CUDA tensors uses the library's grouped send / recv kernel (queued until the first wait, so an isend + irecv pair
@@ -32,6 +32,9 @@ from ..ops import coll
 
 BACKEND_NAME = "b200coll"
 _FAST_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
+# fp8 reductions: sum / avg on the fused kernels (fp32 accumulation, saturating result), min / max / product on the generic kernel. Not in
+# _FAST_DTYPES: all-gather, all-to-all and broadcast of fp8 keep moving raw words (bit-exact, never the Lamport path).
+_FP8_DTYPES = (torch.float8_e4m3fn, torch.float8_e5m2)
 
 
 class _Work(dist._Work):
@@ -83,6 +86,11 @@ def _fast(t: torch.Tensor) -> bool:
     return t.is_cuda and t.is_contiguous() and t.dtype in _FAST_DTYPES and t.data_ptr() % 16 == 0 and t.numel() > 0
 
 
+def _rs_direct(t: torch.Tensor) -> bool:
+    """Reduce-scatter runs on the library directly for the fast dtypes and for fp8 (sum / avg)."""
+    return _fast(t) or (t.is_cuda and t.is_contiguous() and t.dtype in _FP8_DTYPES and t.data_ptr() % 16 == 0 and t.numel() > 0)
+
+
 _GENERIC_DTYPES = (torch.int8, torch.uint8, torch.int32, torch.int64, torch.float64)      # any operator but AVG, on the generic P2P kernel
 
 
@@ -108,7 +116,7 @@ def _red_op(op) -> Optional[int]:
 def _reducible(t: torch.Tensor, op: Optional[int]) -> bool:
     if op is None or not (t.is_cuda and t.is_contiguous() and t.data_ptr() % 16 == 0 and t.numel() > 0):
         return False
-    if t.dtype in _FAST_DTYPES:
+    if t.dtype in _FAST_DTYPES or t.dtype in _FP8_DTYPES:
         return True
     return t.dtype in _GENERIC_DTYPES and op != coll.AVG
 
@@ -353,7 +361,7 @@ class B200CollProcessGroup(dist.ProcessGroup):
 
     def _reduce_scatter_base(self, output, input, opts=None):
         op = _sum_or_avg(opts.reduceOp) if opts is not None else coll.SUM
-        if op is not None and _fast(output) and _fast(input) and output.dtype == input.dtype and (output.numel() * output.element_size()) % 16 == 0 \
+        if op is not None and _rs_direct(output) and _rs_direct(input) and output.dtype == input.dtype and (output.numel() * output.element_size()) % 16 == 0 \
                 and input.numel() == output.numel() * self._size:
             with self._ordered(self):
                 self.comm.reduce_scatter(input.view(-1), output.view(-1), op=op)
