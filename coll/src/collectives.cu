@@ -77,6 +77,59 @@ static b200collResult_t dispatch_types(b200collDataType_t in, b200collDataType_t
 template <typename T> constexpr bool kMcKernels = !IsFp8<T>::value;
 static bool is_fp8(b200collDataType_t t) { return t == b200collFloat8e4m3 || t == b200collFloat8e5m2; }
 
+// f(std::true_type{}) launches a kernel's multicast variant, f(std::false_type{}) its P2P one; only an input type with multicast
+// kernels ever reaches the former.
+template <typename InT, typename F>
+static auto with_mc(bool mc, F&& f) {
+  if constexpr (kMcKernels<InT>) { if (mc) return f(std::true_type{}); }
+  return f(std::false_type{});
+}
+
+// What the algorithm of a fused collective depends on besides the communicator (ranks, multicast, forced algorithm, tuner table).
+struct CallFacts {
+  b200collOp_t op;
+  size_t bytes;                  // as the tuner sees them
+  b200collDataType_t in_dtype;
+  bool sym_in, sym_out;          // inside the symmetric arena
+  bool inplace, same_size;       // send == recv; input and output elements of equal size
+};
+
+// The algorithm a call runs: the forced algorithm or the tuner's pick, moved to one that can serve the call. b200collAlgoAuto means
+// that no all-reduce algorithm can run on these buffers and the call is staged; `staging` then asks for the algorithm that runs
+// between the two staging halves (symmetric, not in place), which follows no pick.
+static b200collAlgo_t resolve_algo(const b200collComm* c, const CallFacts& f, bool staging = false) {
+  const bool mc = c->nvls && !is_fp8(f.in_dtype);      // no multicast kernel for an fp8 input (above)
+  b200collAlgo_t a = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(f.op, f.bytes, c->nranks, c->nvls);
+  switch (f.op) {
+    case b200collOpAllReduce: {
+      auto feasible = [&](b200collAlgo_t x) {
+        switch (x) {
+          case b200collAlgoLL: return f.bytes <= kLLOneShotMaxBytes;
+          case b200collAlgoLL2: return f.same_size && f.bytes <= kLLOneShotMaxBytes * (size_t)c->nranks;
+          case b200collAlgoOneShot: return f.sym_in && !f.inplace;
+          case b200collAlgoTwoShot: return f.sym_in && f.sym_out;
+          case b200collAlgoNvls: return mc && f.sym_in && f.sym_out;
+          default: return false;
+        }
+      };
+      if (!staging && feasible(a)) return a;
+      for (b200collAlgo_t x : {b200collAlgoNvls, b200collAlgoTwoShot, b200collAlgoOneShot, b200collAlgoLL, b200collAlgoLL2})
+        if (feasible(x) && !(x == b200collAlgoNvls && c->nranks == 2)) return x;
+      return b200collAlgoAuto;
+    }
+    case b200collOpAllGather:
+    case b200collOpReduceScatter:
+      if (a == b200collAlgoLL2) a = b200collAlgoLL;
+      if ((a == b200collAlgoLL && f.bytes > kLLOneShotMaxBytes) || (a == b200collAlgoNvls && !mc) || a == b200collAlgoOneShot || a == b200collAlgoCopy) a = b200collAlgoTwoShot;
+      return a;
+    case b200collOpAllToAll:
+      if (a == b200collAlgoLL2) a = b200collAlgoLL;
+      return (a == b200collAlgoLL && f.bytes <= kLLOneShotMaxBytes) ? b200collAlgoLL : b200collAlgoTwoShot;
+    default:                     // broadcast, reduce: multimem or P2P
+      return (a == b200collAlgoNvls && mc) ? b200collAlgoNvls : b200collAlgoTwoShot;
+  }
+}
+
 #define LAUNCH_CHECK(c)                                                                                  \
   do {                                                                                                   \
     cudaError_t e__ = cudaGetLastError();                                                                \
@@ -115,19 +168,11 @@ static void launch_k_smem(void (*kernel)(KArgs...), int blocks, int threads, siz
     attr.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &attr; cfg.numAttrs = 1;
   }
-  (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+  (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // the error is picked up by LAUNCH_CHECK's cudaGetLastError
 }
 template <typename... KArgs, typename... Args>
 static void launch_k(void (*kernel)(KArgs...), int blocks, int threads, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)blocks); cfg.blockDim = dim3((unsigned)threads); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-  cudaLaunchAttribute attr;
-  if (pdl_enabled()) {
-    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr.val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = &attr; cfg.numAttrs = 1;
-  }
-  (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // the error is picked up by LAUNCH_CHECK's cudaGetLastError
+  launch_k_smem(kernel, blocks, threads, 0, st, std::forward<Args>(args)...);
 }
 
 // Pick the smallest block size that still covers `vecs` with <= max_ctas blocks (small work spreads over more SMs),
@@ -150,15 +195,24 @@ static Grid pick_grid(const b200collComm* c, int kind, size_t vecs, int unroll) 
 }
 
 static size_t arena_off(b200collComm* c, const void* p) { return reinterpret_cast<CUdeviceptr>(p) - c->peer_va[c->rank]; }
-static char* stage_ptr(b200collComm* c, int half) { return reinterpret_cast<char*>(c->peer_va[c->rank]) + kOffStage + (size_t)half * kStageHalfBytes; }
+
+b200collResult_t copy_rows(char* dst, size_t dst_pitch, const char* src, size_t src_pitch, size_t bytes, int rows, cudaStream_t st) {
+  for (int r = 0; r < rows; r++) {
+    const cudaError_t e = cudaMemcpyAsync(dst + (size_t)r * dst_pitch, src + (size_t)r * src_pitch, bytes, cudaMemcpyDeviceToDevice, st);
+    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
+  }
+  return b200collSuccess;
+}
 
 static bool aligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
 static size_t out_align(size_t in_sz, size_t out_sz) { return std::min<size_t>(16, 16 / in_sz * out_sz); }
 
 static b200collResult_t check_common(b200collComm* c, const void* send, void* recv, const b200collEpilogue* ep) {
   if (!c || !send || !recv || !ep) { set_last_error("null argument"); return b200collInvalidArgument; }
-  auto fused = [](b200collDataType_t t) { return ((int)t >= 0 && (int)t <= (int)b200collFloat8e4m3) || t == b200collFloat8e5m2; };
-  if (!fused(ep->in_dtype) || !fused(ep->out_dtype)) { set_last_error("bad dtype (fp32 / fp16 / bf16 / fp8 e4m3 / fp8 e5m2 in and out; integer and fp64 payloads: reductions take the generic path, data movement takes them as words)"); return b200collInvalidArgument; }
+  if (dispatch_types(ep->in_dtype, ep->out_dtype, [](auto, auto) { return b200collSuccess; }) != b200collSuccess) {
+    set_last_error("unsupported (in_dtype, out_dtype) pair (fp32 / fp16 / bf16 / fp8 e4m3 / fp8 e5m2 in and out; integer and fp64 payloads: reductions take the generic path, data movement takes them as words)");
+    return b200collInvalidArgument;
+  }
   const size_t is = b200collTypeSize(ep->in_dtype), os = b200collTypeSize(ep->out_dtype);
   if (!aligned(send, 16) || !aligned(recv, out_align(is, os))) { set_last_error("send must be 16-byte aligned and recv aligned to one output vector"); return b200collInvalidArgument; }
   if (c->fault_host && *const_cast<volatile uint32_t*>(&c->fault_host->code) != 0) { set_last_error("communicator is poisoned by an earlier watchdog fault"); return b200collRemoteError; }
@@ -273,49 +327,36 @@ static b200collResult_t launch_ll(b200collComm* c, b200collOp_t op, const void* 
     const size_t nv = (count + E - 1) / E;
     Grid g = pick_grid(c, kShapeLL, nv, 1);
     const InT* in = static_cast<const InT*>(send); OutT* out = static_cast<OutT*>(recv);
-    const bool mc = c->nvls && kMcKernels<InT>;
     struct PdlScope { PdlScope(bool v) { t_pdl_small = v; } ~PdlScope() { t_pdl_small = false; } } pdl_scope(count * sizeof(InT) <= pdl_max_bytes());
-    switch (op) {
-      case b200collOpAllReduce:
-        if (mc) { if constexpr (kMcKernels<InT>) launch_k(k_ll<InT, OutT, false, true, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); }
-        else launch_k(k_ll<InT, OutT, false, true, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
-        break;
-      case b200collOpAllGather:
-        if (mc) { if constexpr (kMcKernels<InT>) launch_k(k_ll<InT, OutT, false, false, true>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); }
-        else launch_k(k_ll<InT, OutT, false, false, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
-        break;
-      case b200collOpReduceScatter:
-        launch_k(k_ll<InT, OutT, true, true, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
-        break;
-      default:
-        launch_k(k_ll<InT, OutT, true, false, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
-        break;
-    }
+    if (op == b200collOpAllReduce)
+      with_mc<InT>(c->nvls, [&](auto mc) { launch_k(k_ll<InT, OutT, false, true, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); });
+    else if (op == b200collOpAllGather)
+      with_mc<InT>(c->nvls, [&](auto mc) { launch_k(k_ll<InT, OutT, false, false, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op); });
+    else if (op == b200collOpReduceScatter)
+      launch_k(k_ll<InT, OutT, true, true, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
+    else
+      launch_k(k_ll<InT, OutT, true, false, false>, g.blocks, g.threads, st, c->dev, in, out, count, scale, op);
     LAUNCH_CHECK(c);
     return b200collSuccess;
   });
 }
 
-// Two-shot Lamport all-reduce (same-size in/out types only; any local pointers, in-place allowed).
-template <typename InT, typename OutT>
-static b200collResult_t launch_ll2_typed(b200collComm* c, const void* send, void* recv, size_t count, float scale, cudaStream_t st) {
-  constexpr int E = Epv<InT>::value;
-  const size_t nslice = ((count + E - 1) / E + c->nranks - 1) / c->nranks;
-  Grid g = pick_grid(c, kShapeLL, nslice, 1);
-  if (c->nvls && kMcKernels<InT>) { if constexpr (kMcKernels<InT>) launch_k(k_ll_twoshot<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce); }
-  else launch_k(k_ll_twoshot<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce);
-  LAUNCH_CHECK(c);
-  return b200collSuccess;
-}
+// Two-shot Lamport all-reduce (same in/out type only; any local pointers, in-place allowed).
 static b200collResult_t launch_ll2(b200collComm* c, const void* send, void* recv, size_t count, const b200collEpilogue* ep, float scale, cudaStream_t st) {
-  const b200collDataType_t i = ep->in_dtype, o = ep->out_dtype;
-  if (i == b200collFloat32 && o == b200collFloat32) return launch_ll2_typed<float, float>(c, send, recv, count, scale, st);
-  if (i == b200collBfloat16 && o == b200collBfloat16) return launch_ll2_typed<bf16, bf16>(c, send, recv, count, scale, st);
-  if (i == b200collFloat16 && o == b200collFloat16) return launch_ll2_typed<__half, __half>(c, send, recv, count, scale, st);
-  if (i == b200collFloat8e4m3 && o == b200collFloat8e4m3) return launch_ll2_typed<f8, f8>(c, send, recv, count, scale, st);
-  if (i == b200collFloat8e5m2 && o == b200collFloat8e5m2) return launch_ll2_typed<f8e5, f8e5>(c, send, recv, count, scale, st);
-  set_last_error("two-shot LL needs in_dtype == out_dtype");
-  return b200collInvalidArgument;
+  return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
+    using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
+    if constexpr (std::is_same_v<InT, OutT>) {
+      constexpr int E = Epv<InT>::value;
+      const size_t nslice = ((count + E - 1) / E + c->nranks - 1) / c->nranks;
+      Grid g = pick_grid(c, kShapeLL, nslice, 1);
+      with_mc<InT>(c->nvls, [&](auto mc) { launch_k(k_ll_twoshot<InT, OutT, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(send), static_cast<OutT*>(recv), count, scale, b200collOpAllReduce); });
+      LAUNCH_CHECK(c);
+      return b200collSuccess;
+    } else {
+      set_last_error("two-shot LL needs in_dtype == out_dtype");
+      return b200collInvalidArgument;
+    }
+  });
 }
 
 // ------------------------------------------------------------------------------------------------ all-reduce on symmetric buffers
@@ -332,23 +373,18 @@ static b200collResult_t ar_symmetric(b200collComm* c, b200collAlgo_t algo, const
     } else if (algo == b200collAlgoTwoShot) {
       Grid g = pick_grid(c, kShapeP2p, nvec / c->nranks + 1, 2);
       launch_k(k_ar_twoshot<InT, OutT>, g.blocks, g.threads, st, c->dev, in_off, arena_off(c, recv), count, scale, b200collOpAllReduce);
-    } else if constexpr (!kMcKernels<InT>) {
-      set_last_error("no NVLS all-reduce kernel for fp8 inputs");
-      return b200collInternalError;
     } else {
-      static const int forced_u = [] { const char* e = getenv("B200COLL_NVLS_UNROLL"); return e ? atoi(e) : 0; }();
-      const size_t slice = nvec / c->nranks + 1;
-      Grid g = pick_grid(c, kShapeNvls, slice, 4);
-      // U=1 (more, thinner passes so multimem.st overlaps the next ld_reduce) was measured on 8xB200 and LOST to U=4 at every
-      // mid size (512 KiB: 20.1 vs 16.0 us, 8 MiB: 38.7 vs 33.9 us): it needs 4x the CTAs, and every extra CTA adds 8 flag
-      // stores + a membar.sys to both barriers. U=4 ships; B200COLL_NVLS_UNROLL=1 keeps the variant reachable.
-      const int u = forced_u ? forced_u : 4;
-      if (u == 1) {
-        g = pick_grid(c, kShapeNvls, slice, 1);
-        launch_k(k_ar_nvls<InT, OutT, 1>, g.blocks, g.threads, st, c->dev, in_off, arena_off(c, recv), count, scale, identity, b200collOpAllReduce);
-      } else {
-        launch_k(k_ar_nvls<InT, OutT, 4>, g.blocks, g.threads, st, c->dev, in_off, arena_off(c, recv), count, scale, identity, b200collOpAllReduce);
-      }
+      // U=4 vectors in flight per thread. U=1 (more, thinner passes so multimem.st overlaps the next ld_reduce) was measured on
+      // 8xB200 and lost to U=4 at every mid size (512 KiB: 20.1 vs 16.0 us, 8 MiB: 38.7 vs 33.9 us): it needs 4x the CTAs, and every
+      // extra CTA adds 8 flag stores + a membar.sys to both barriers.
+      const bool launched = with_mc<InT>(true, [&](auto mc) {
+        if constexpr (decltype(mc)::value) {
+          Grid g = pick_grid(c, kShapeNvls, nvec / c->nranks + 1, 4);
+          launch_k(k_ar_nvls<InT, OutT, 4>, g.blocks, g.threads, st, c->dev, in_off, arena_off(c, recv), count, scale, identity, b200collOpAllReduce);
+        }
+        return decltype(mc)::value;
+      });
+      if (!launched) { set_last_error("no NVLS all-reduce kernel for fp8 inputs"); return b200collInternalError; }
     }
     LAUNCH_CHECK(c);
     return b200collSuccess;
@@ -519,22 +555,8 @@ b200collResult_t b200collAllReduce(const void* send, void* recv, size_t count, c
   if (inplace && is != os) { set_last_error("in-place all-reduce needs in_dtype and out_dtype of equal size"); return b200collInvalidArgument; }
   if (c->nranks == 1) { account(c, b200collOpAllReduce, bytes, b200collAlgoCopy); return copy_scale(c, send, recv, count, ep, scale, st); }
   const bool sym_in = b200collIsSymmetric(c, send, bytes), sym_out = b200collIsSymmetric(c, recv, count * os);
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpAllReduce, bytes, c->nranks, c->nvls);
-  auto feasible = [&](b200collAlgo_t a) {
-    switch (a) {
-      case b200collAlgoLL: return bytes <= kLLOneShotMaxBytes;
-      case b200collAlgoLL2: return is == os && bytes <= kLLOneShotMaxBytes * (size_t)c->nranks;
-      case b200collAlgoOneShot: return sym_in && !inplace;
-      case b200collAlgoTwoShot: return sym_in && sym_out;
-      case b200collAlgoNvls: return c->nvls && sym_in && sym_out && !is_fp8(ep->in_dtype);   // see kMcKernels
-      default: return false;
-    }
-  };
-  if (!feasible(algo)) {
-    algo = b200collAlgoAuto;
-    for (b200collAlgo_t a : {b200collAlgoNvls, b200collAlgoTwoShot, b200collAlgoOneShot, b200collAlgoLL, b200collAlgoLL2})
-      if (feasible(a) && !(a == b200collAlgoNvls && c->nranks == 2)) { algo = a; break; }
-  }
+  CallFacts f = {b200collOpAllReduce, bytes, ep->in_dtype, sym_in, sym_out, inplace, is == os};
+  const b200collAlgo_t algo = resolve_algo(c, f);
   if (algo == b200collAlgoLL) { account(c, b200collOpAllReduce, bytes, algo); return launch_ll(c, b200collOpAllReduce, send, recv, count, ep, scale, st); }
   if (algo == b200collAlgoLL2) { account(c, b200collOpAllReduce, bytes, algo); return launch_ll2(c, send, recv, count, ep, scale, st); }
   if (algo != b200collAlgoAuto) {
@@ -543,21 +565,13 @@ b200collResult_t b200collAllReduce(const void* send, void* recv, size_t count, c
     account(c, b200collOpAllReduce, bytes, algo);
     return ar_symmetric(c, algo, send, recv, count, ep, scale, st);
   }
-  // ---- staged: buffers outside the arena and too big for LL. Chunk through the two staging halves.
-  c->stats.staged_calls++;
-  b200collAlgo_t inner = (c->nvls && c->nranks > 2 && !is_fp8(ep->in_dtype)) ? b200collAlgoNvls : b200collAlgoTwoShot;
-  const size_t chunk = std::min(kStageHalfBytes / is, kStageHalfBytes / os) / 64 * 64;
-  for (size_t done = 0; done < count; done += chunk) {
-    const size_t n = std::min(chunk, count - done);
-    cudaError_t e = cudaMemcpyAsync(stage_ptr(c, 0), static_cast<const char*>(send) + done * is, n * is, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
+  // ---- staged: buffers outside the arena and too big for LL
+  f.sym_in = f.sym_out = true; f.inplace = false;
+  const b200collAlgo_t inner = resolve_algo(c, f, /*staging=*/true);
+  return run_staged(c, count, stage_chunk(std::max(is, os), 1), {send, is, 1}, {recv, os, 1}, st, [&](size_t, size_t n) {
     account(c, b200collOpAllReduce, n * is, inner);
-    rc = ar_symmetric(c, inner, stage_ptr(c, 0), stage_ptr(c, 1), n, ep, scale, st);
-    if (rc != b200collSuccess) return rc;
-    e = cudaMemcpyAsync(static_cast<char*>(recv) + done * os, stage_ptr(c, 1), n * os, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-  }
-  return b200collSuccess;
+    return ar_symmetric(c, inner, stage_ptr(c, 0), stage_ptr(c, 1), n, ep, scale, st);
+  });
 }
 
 b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcount, const b200collEpilogue* ep, b200collComm_t c, b200collStream_t stream) {
@@ -571,11 +585,7 @@ b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcoun
   if (c->nranks == 1) { account(c, b200collOpAllGather, bytes, b200collAlgoCopy); return copy_scale(c, send, recv, sendcount, ep, scale, st); }
   if (sendcount % (16 / is) != 0) { set_last_error("all-gather sendcount must be a multiple of 16 bytes / sizeof(in_dtype)"); return b200collInvalidArgument; }
   const bool sym_out = b200collIsSymmetric(c, recv, (size_t)c->nranks * sendcount * os);
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpAllGather, bytes, c->nranks, c->nvls);
-  if (algo == b200collAlgoOneShot) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoLL2) algo = b200collAlgoLL;
-  if (algo == b200collAlgoLL && bytes > kLLOneShotMaxBytes) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoNvls && (!c->nvls || is_fp8(ep->in_dtype))) algo = b200collAlgoTwoShot;   // fp8: see kMcKernels
+  const b200collAlgo_t algo = resolve_algo(c, {b200collOpAllGather, bytes, ep->in_dtype});
   if (algo == b200collAlgoLL) { account(c, b200collOpAllGather, bytes, algo); return launch_ll(c, b200collOpAllGather, send, recv, sendcount, ep, scale, st); }
   const int identity = (ep->in_dtype == ep->out_dtype && scale == 1.0f) ? 1 : 0;
   auto push = [&](const void* s, void* r, size_t n) -> b200collResult_t {
@@ -583,8 +593,7 @@ b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcoun
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeNvls : kShapeP2p, n / Epv<InT>::value, 4);
-      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_ag_push<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather); }
-      else launch_k(k_ag_push<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather);
+      with_mc<InT>(algo == b200collAlgoNvls, [&](auto mc) { launch_k(k_ag_push<InT, OutT, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r), n, scale, identity, b200collOpAllGather); });
       LAUNCH_CHECK(c);
       return b200collSuccess;
     });
@@ -602,18 +611,8 @@ b200collResult_t b200collAllGather(const void* send, void* recv, size_t sendcoun
   }
   if (sym_out) return push(send, recv, sendcount);
   // staged: gather chunks into staging half 1 laid out [nranks][chunk], then scatter locally into recv
-  c->stats.staged_calls++;
-  const size_t chunk = (kStageHalfBytes / os / c->nranks) / 64 * 64;
-  for (size_t done = 0; done < sendcount; done += chunk) {
-    const size_t n = std::min(chunk, sendcount - done);
-    rc = push(static_cast<const char*>(send) + done * is, stage_ptr(c, 1), n);
-    if (rc != b200collSuccess) return rc;
-    for (int r = 0; r < c->nranks; r++) {
-      cudaError_t e = cudaMemcpyAsync(static_cast<char*>(recv) + ((size_t)r * sendcount + done) * os, stage_ptr(c, 1) + (size_t)r * n * os, n * os, cudaMemcpyDeviceToDevice, st);
-      if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-    }
-  }
-  return b200collSuccess;
+  return run_staged(c, sendcount, stage_chunk(os, c->nranks), {}, {recv, os, c->nranks}, st,
+                    [&](size_t done, size_t n) { return push(static_cast<const char*>(send) + done * is, stage_ptr(c, 1), n); });
 }
 
 b200collResult_t b200collReduceScatter(const void* send, void* recv, size_t recvcount, const b200collEpilogue* ep, b200collRedOp_t rop, b200collComm_t c, b200collStream_t stream) {
@@ -629,19 +628,14 @@ b200collResult_t b200collReduceScatter(const void* send, void* recv, size_t recv
   if (c->nranks == 1) { account(c, b200collOpReduceScatter, bytes, b200collAlgoCopy); return copy_scale(c, send, recv, recvcount, ep, scale, st); }
   if (recvcount % (16 / is) != 0) { set_last_error("reduce-scatter recvcount must be a multiple of 16 bytes / sizeof(in_dtype)"); return b200collInvalidArgument; }
   const bool sym_in = b200collIsSymmetric(c, send, (size_t)c->nranks * bytes);
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpReduceScatter, bytes, c->nranks, c->nvls);
-  if (algo == b200collAlgoOneShot) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoLL2) algo = b200collAlgoLL;
-  if (algo == b200collAlgoLL && bytes > kLLOneShotMaxBytes) algo = b200collAlgoTwoShot;
-  if (algo == b200collAlgoNvls && (!c->nvls || is_fp8(ep->in_dtype))) algo = b200collAlgoTwoShot;   // fp8: see kMcKernels
+  const b200collAlgo_t algo = resolve_algo(c, {b200collOpReduceScatter, bytes, ep->in_dtype});
   if (algo == b200collAlgoLL) { account(c, b200collOpReduceScatter, bytes, algo); return launch_ll(c, b200collOpReduceScatter, send, recv, recvcount, ep, scale, st); }
   auto pull = [&](const void* s_slice_of_mine, void* r, size_t n) -> b200collResult_t {
     account(c, b200collOpReduceScatter, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeNvlsRs : kShapeP2p, n / Epv<InT>::value, 2);
-      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_pull_reduce<InT, OutT, false, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter); }
-      else launch_k(k_pull_reduce<InT, OutT, false, false>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter);
+      with_mc<InT>(algo == b200collAlgoNvls, [&](auto mc) { launch_k(k_pull_reduce<InT, OutT, false, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, arena_off(c, s_slice_of_mine), static_cast<OutT*>(r), n, scale, b200collOpReduceScatter); });
       LAUNCH_CHECK(c);
       return b200collSuccess;
     });
@@ -652,18 +646,8 @@ b200collResult_t b200collReduceScatter(const void* send, void* recv, size_t recv
     return pull(static_cast<const char*>(send) + (size_t)c->rank * bytes, recv, recvcount);
   }
   // staged: copy chunk j of every slice into staging half 0 laid out [nranks][chunk]; each rank pulls its row
-  c->stats.staged_calls++;
-  const size_t chunk = (kStageHalfBytes / is / c->nranks) / 64 * 64;
-  for (size_t done = 0; done < recvcount; done += chunk) {
-    const size_t n = std::min(chunk, recvcount - done);
-    for (int r = 0; r < c->nranks; r++) {
-      cudaError_t e = cudaMemcpyAsync(stage_ptr(c, 0) + (size_t)r * n * is, static_cast<const char*>(send) + ((size_t)r * recvcount + done) * is, n * is, cudaMemcpyDeviceToDevice, st);
-      if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-    }
-    rc = pull(stage_ptr(c, 0) + (size_t)c->rank * n * is, static_cast<char*>(recv) + done * os, n);
-    if (rc != b200collSuccess) return rc;
-  }
-  return b200collSuccess;
+  return run_staged(c, recvcount, stage_chunk(is, c->nranks), {send, is, c->nranks}, {}, st,
+                    [&](size_t done, size_t n) { return pull(stage_ptr(c, 0) + (size_t)c->rank * n * is, static_cast<char*>(recv) + done * os, n); });
 }
 
 // symmetric: every rank moves the same amount, so the grid may follow the work. Otherwise (all-to-all-v: each rank only knows its own
@@ -701,9 +685,7 @@ b200collResult_t b200collAllToAll(const void* send, void* recv, size_t count, co
   if (send == recv) { set_last_error("in-place all-to-all is not supported"); return b200collInvalidUsage; }
   const size_t E = 16 / is;
   if (count % E != 0) { set_last_error("all-to-all count must be a multiple of 16 bytes / sizeof(in_dtype)"); return b200collInvalidArgument; }
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpAllToAll, bytes, c->nranks, c->nvls);
-  if (algo == b200collAlgoLL2) algo = b200collAlgoLL;
-  if (algo != b200collAlgoLL || bytes > kLLOneShotMaxBytes) algo = b200collAlgoTwoShot;
+  const b200collAlgo_t algo = resolve_algo(c, {b200collOpAllToAll, bytes, ep->in_dtype});
   if (algo == b200collAlgoLL) { account(c, b200collOpAllToAll, bytes * c->nranks, algo); return launch_ll(c, b200collOpAllToAll, send, recv, count, ep, ep->scale, st); }
   const bool sym_out = b200collIsSymmetric(c, recv, (size_t)c->nranks * count * os);
   auto run = [&](const void* s, size_t s_stride_elems, void* r_sym, size_t n) -> b200collResult_t {
@@ -731,18 +713,8 @@ b200collResult_t b200collAllToAll(const void* send, void* recv, size_t count, co
     return launch_bulk(c, a, true, b200collOpAllToAll, st);
   }
   if (sym_out) return run(send, count, recv, count);
-  c->stats.staged_calls++;
-  const size_t chunk = (kStageHalfBytes / os / c->nranks) / 64 * 64;
-  for (size_t done = 0; done < count; done += chunk) {
-    const size_t n = std::min(chunk, count - done);
-    rc = run(static_cast<const char*>(send) + done * is, count, stage_ptr(c, 1), n);
-    if (rc != b200collSuccess) return rc;
-    for (int r = 0; r < c->nranks; r++) {
-      cudaError_t e = cudaMemcpyAsync(static_cast<char*>(recv) + ((size_t)r * count + done) * os, stage_ptr(c, 1) + (size_t)r * n * os, n * os, cudaMemcpyDeviceToDevice, st);
-      if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-    }
-  }
-  return b200collSuccess;
+  return run_staged(c, count, stage_chunk(os, c->nranks), {}, {recv, os, c->nranks}, st,
+                    [&](size_t done, size_t n) { return run(static_cast<const char*>(send) + done * is, count, stage_ptr(c, 1), n); });
 }
 
 b200collResult_t b200collAllToAllv(const void* send, void* recv, size_t row_elems, const int64_t* send_rows, const int64_t* send_row_off,
@@ -790,16 +762,14 @@ b200collResult_t b200collBroadcast(const void* send, void* recv, size_t count, c
   const float scale = ep->scale;
   if (c->nranks == 1) { account(c, b200collOpBroadcast, count * is, b200collAlgoCopy); return copy_scale(c, send, recv, count, ep, scale, st); }
   if (send == recv && is != os) { set_last_error("in-place broadcast needs in_dtype and out_dtype of equal size"); return b200collInvalidArgument; }
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpBroadcast, count * is, c->nranks, c->nvls);
-  if (algo != b200collAlgoNvls || !c->nvls || is_fp8(ep->in_dtype)) algo = b200collAlgoTwoShot;     // two families only: multimem.st or P2P push
+  const b200collAlgo_t algo = resolve_algo(c, {b200collOpBroadcast, count * is, ep->in_dtype});
   const int identity = (ep->in_dtype == ep->out_dtype && scale == 1.0f) ? 1 : 0;
   auto push = [&](const void* s, void* r_sym, size_t n) -> b200collResult_t {
     account(c, b200collOpBroadcast, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeRooted : kShapeP2p, std::max<size_t>(1, n / Epv<InT>::value), 4);
-      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_bcast<InT, OutT, true>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast); }
-      else launch_k(k_bcast<InT, OutT, false>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast);
+      with_mc<InT>(algo == b200collAlgoNvls, [&](auto mc) { launch_k(k_bcast<InT, OutT, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, static_cast<const InT*>(s), arena_off(c, r_sym), n, scale, identity, root, b200collOpBroadcast); });
       LAUNCH_CHECK(c);
       return b200collSuccess;
     });
@@ -813,16 +783,8 @@ b200collResult_t b200collBroadcast(const void* send, void* recv, size_t count, c
   }
   if (b200collIsSymmetric(c, recv, count * os)) return push(send, recv, count);
   // staged: the root pushes a chunk into everybody's staging half 1, each rank copies it out locally
-  c->stats.staged_calls++;
-  const size_t chunk = std::min(kStageHalfBytes / is, kStageHalfBytes / os) / 64 * 64;
-  for (size_t done = 0; done < count; done += chunk) {
-    const size_t n = std::min(chunk, count - done);
-    rc = push(static_cast<const char*>(send) + done * is, stage_ptr(c, 1), n);
-    if (rc != b200collSuccess) return rc;
-    cudaError_t e = cudaMemcpyAsync(static_cast<char*>(recv) + done * os, stage_ptr(c, 1), n * os, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-  }
-  return b200collSuccess;
+  return run_staged(c, count, stage_chunk(std::max(is, os), 1), {}, {recv, os, 1}, st,
+                    [&](size_t done, size_t n) { return push(static_cast<const char*>(send) + done * is, stage_ptr(c, 1), n); });
 }
 
 b200collResult_t b200collReduce(const void* send, void* recv, size_t count, const b200collEpilogue* ep, b200collRedOp_t rop, int root, b200collComm_t c, b200collStream_t stream) {
@@ -841,31 +803,21 @@ b200collResult_t b200collReduce(const void* send, void* recv, size_t count, cons
   const float scale = ep->scale * (rop == b200collAvg ? 1.0f / (float)c->nranks : 1.0f);
   if (c->nranks == 1) { account(c, b200collOpReduce, count * is, b200collAlgoCopy); return copy_scale(c, send, recv, count, ep, scale, st); }
   if (send == recv && is != os) { set_last_error("in-place reduce needs in_dtype and out_dtype of equal size"); return b200collInvalidArgument; }
-  b200collAlgo_t algo = c->forced_algo != b200collAlgoAuto ? c->forced_algo : b200collTunerPick(b200collOpReduce, count * is, c->nranks, c->nvls);
-  if (algo != b200collAlgoNvls || !c->nvls || is_fp8(ep->in_dtype)) algo = b200collAlgoTwoShot;     // multimem.ld_reduce by the root, or the root pulls from every peer
+  const b200collAlgo_t algo = resolve_algo(c, {b200collOpReduce, count * is, ep->in_dtype});
   auto pull = [&](const void* s_sym, void* r, size_t n) -> b200collResult_t {
     account(c, b200collOpReduce, n * is, algo);
     return dispatch_types(ep->in_dtype, ep->out_dtype, [&](auto ti, auto to) -> b200collResult_t {
       using InT = typename decltype(ti)::type; using OutT = typename decltype(to)::type;
       Grid g = pick_grid(c, algo == b200collAlgoNvls ? kShapeRooted : kShapeP2p, std::max<size_t>(1, n / Epv<InT>::value), algo == b200collAlgoNvls ? 4 : 2);
-      if (algo == b200collAlgoNvls) { if constexpr (kMcKernels<InT>) launch_k(k_reduce_root<InT, OutT, true>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce); }
-      else launch_k(k_reduce_root<InT, OutT, false>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce);
+      with_mc<InT>(algo == b200collAlgoNvls, [&](auto mc) { launch_k(k_reduce_root<InT, OutT, decltype(mc)::value>, g.blocks, g.threads, st, c->dev, arena_off(c, s_sym), static_cast<OutT*>(r), n, scale, root, b200collOpReduce); });
       LAUNCH_CHECK(c);
       return b200collSuccess;
     });
   };
   if (b200collIsSymmetric(c, send, count * is)) return pull(send, recv, count);
   // staged: every rank copies a chunk of its send buffer into staging half 0, the root reduces the chunk into recv
-  c->stats.staged_calls++;
-  const size_t chunk = std::min(kStageHalfBytes / is, kStageHalfBytes / os) / 64 * 64;
-  for (size_t done = 0; done < count; done += chunk) {
-    const size_t n = std::min(chunk, count - done);
-    cudaError_t e = cudaMemcpyAsync(stage_ptr(c, 0), static_cast<const char*>(send) + done * is, n * is, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-    rc = pull(stage_ptr(c, 0), static_cast<char*>(recv) + done * os, n);
-    if (rc != b200collSuccess) return rc;
-  }
-  return b200collSuccess;
+  return run_staged(c, count, stage_chunk(std::max(is, os), 1), {send, is, 1}, {}, st,
+                    [&](size_t done, size_t n) { return pull(stage_ptr(c, 0), static_cast<char*>(recv) + done * os, n); });
 }
 
 b200collResult_t b200collGroupStart(void) { g_group_depth++; return b200collSuccess; }

@@ -4,6 +4,7 @@
 #include <sched.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 #include <map>
 #include <memory>
@@ -108,15 +109,34 @@ struct b200collComm {
 
 namespace b200coll {
 
-struct LaunchPlan {
-  b200collAlgo_t algo;
-  int blocks;
-  int threads;
-};
-
-// tuner.cc
 void stats_page_publish(b200collComm* c);   // comm.cu
-int tuner_blocks(b200collOp_t op, b200collAlgo_t algo, size_t work_vecs, int max_ctas, int unroll);
+
+// ---- staging (collectives.cu, generic.cu): buffers outside the symmetric arena go through the two staging halves, chunk by chunk.
+// A chunk of n elements that starts at element `done` is copied into staging half 0 as `rows` rows (row r: elements
+// [r * count + done, + n) of the user buffer -> [r * n, + n) of the half), the kernel runs, and the result is copied out of
+// staging half 1 the same way. A null buffer skips that copy: the kernel reads or writes the user buffer itself.
+struct StageIn { const void* buf; size_t elem; int rows; };
+struct StageOut { void* buf; size_t elem; int rows; };
+
+inline char* stage_ptr(b200collComm* c, int half) { return reinterpret_cast<char*>(c->peer_va[c->rank]) + kOffStage + (size_t)half * kStageHalfBytes; }
+// elements per chunk when `rows` rows of `elem`-byte elements share one staging half
+inline size_t stage_chunk(size_t elem, int rows) { return kStageHalfBytes / elem / rows / 64 * 64; }
+// `rows` device-to-device copies of `bytes` each, row r from src + r * src_pitch to dst + r * dst_pitch
+b200collResult_t copy_rows(char* dst, size_t dst_pitch, const char* src, size_t src_pitch, size_t bytes, int rows, cudaStream_t st);
+
+template <typename F>
+b200collResult_t run_staged(b200collComm* c, size_t count, size_t chunk, StageIn in, StageOut out, cudaStream_t st, F&& kernel) {
+  c->stats.staged_calls++;
+  for (size_t done = 0; done < count; done += chunk) {
+    const size_t n = std::min(chunk, count - done);
+    b200collResult_t rc = b200collSuccess;
+    if (in.buf) rc = copy_rows(stage_ptr(c, 0), n * in.elem, static_cast<const char*>(in.buf) + done * in.elem, count * in.elem, n * in.elem, in.rows, st);
+    if (rc == b200collSuccess) rc = kernel(done, n);
+    if (rc == b200collSuccess && out.buf) rc = copy_rows(static_cast<char*>(out.buf) + done * out.elem, count * out.elem, stage_ptr(c, 1), n * out.elem, n * out.elem, out.rows, st);
+    if (rc != b200collSuccess) return rc;
+  }
+  return b200collSuccess;
+}
 
 // generic.cu
 bool needs_generic(const b200collEpilogue* ep, b200collRedOp_t rop);
@@ -126,8 +146,5 @@ b200collResult_t generic_reduce(b200collComm* c, b200collOp_t which, const void*
 void bind_to_gpu_numa(b200collComm* c, bool allow_bind);   // allow_bind=false: only record the node (in-process groups spanning GPUs)
 void restore_affinity_after_init(b200collComm* c);
 void hostpath_destroy(b200collComm* c);
-
-// collectives.cu
-b200collResult_t launch_fill_sentinel(b200collComm* c, cudaStream_t s);
 
 }  // namespace b200coll

@@ -182,38 +182,18 @@ b200collResult_t generic_reduce(b200collComm* c, b200collOp_t which, const void*
   const bool sym_in = b200collIsSymmetric(c, send, in_elems * es);
   const bool sym_out = b200collIsSymmetric(c, recv, count * es);
   const uint32_t opid = (uint32_t)which;
-  if (sym_in && (which != b200collOpAllReduce || sym_out)) {
-    if (which == b200collOpAllReduce) return dispatch_generic(c, ep->in_dtype, rop, off(send), off(recv), nullptr, count, kModeAllReduce, -1, opid, st);
-    if (which == b200collOpReduceScatter) return dispatch_generic(c, ep->in_dtype, rop, off(send) + (size_t)c->rank * count * es, 0, recv, count, kModeToLocal, -1, opid, st);
-    return dispatch_generic(c, ep->in_dtype, rop, off(send), 0, recv, count, kModeToLocal, root, opid, st);
-  }
+  // m elements of every rank's input at arena offset in_off (all-reduce: result to arena offset out_off, else into out_local)
+  auto launch = [&](size_t in_off, size_t out_off, char* out_local, size_t m) {
+    if (which == b200collOpAllReduce) return dispatch_generic(c, ep->in_dtype, rop, in_off, out_off, nullptr, m, kModeAllReduce, -1, opid, st);
+    if (which == b200collOpReduceScatter) return dispatch_generic(c, ep->in_dtype, rop, in_off + (size_t)c->rank * m * es, 0, out_local, m, kModeToLocal, -1, opid, st);
+    return dispatch_generic(c, ep->in_dtype, rop, in_off, 0, out_local, m, kModeToLocal, root, opid, st);
+  };
+  char* const out = static_cast<char*>(recv);
+  if (sym_in && (which != b200collOpAllReduce || sym_out)) return launch(off(send), off(recv), out, count);
   // staged: chunk through staging half 0 (inputs) and half 1 (all-reduce results)
-  c->stats.staged_calls++;
-  char* const s0 = base + kOffStage;
-  char* const s1 = s0 + kStageHalfBytes;
-  const size_t per = which == b200collOpReduceScatter ? (kStageHalfBytes / es / n) / 64 * 64 : (kStageHalfBytes / es) / 64 * 64;
-  for (size_t done = 0; done < count; done += per) {
-    const size_t m = std::min(per, count - done);
-    cudaError_t e = cudaSuccess;
-    if (which == b200collOpReduceScatter) {
-      for (int r = 0; r < n && e == cudaSuccess; r++)
-        e = cudaMemcpyAsync(s0 + (size_t)r * m * es, static_cast<const char*>(send) + ((size_t)r * count + done) * es, m * es, cudaMemcpyDeviceToDevice, st);
-    } else {
-      e = cudaMemcpyAsync(s0, static_cast<const char*>(send) + done * es, m * es, cudaMemcpyDeviceToDevice, st);
-    }
-    if (e != cudaSuccess) { set_last_error(cudaGetErrorString(e)); return b200collUnhandledCudaError; }
-    b200collResult_t rc;
-    if (which == b200collOpAllReduce) {
-      rc = dispatch_generic(c, ep->in_dtype, rop, kOffStage, kOffStage + kStageHalfBytes, nullptr, m, kModeAllReduce, -1, opid, st);
-      if (rc == b200collSuccess && cudaMemcpyAsync(static_cast<char*>(recv) + done * es, s1, m * es, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = b200collUnhandledCudaError;
-    } else if (which == b200collOpReduceScatter) {
-      rc = dispatch_generic(c, ep->in_dtype, rop, kOffStage + (size_t)c->rank * m * es, 0, static_cast<char*>(recv) + done * es, m, kModeToLocal, -1, opid, st);
-    } else {
-      rc = dispatch_generic(c, ep->in_dtype, rop, kOffStage, 0, static_cast<char*>(recv) + done * es, m, kModeToLocal, root, opid, st);
-    }
-    if (rc != b200collSuccess) return rc;
-  }
-  return b200collSuccess;
+  const int rows = which == b200collOpReduceScatter ? n : 1;
+  return run_staged(c, count, stage_chunk(es, rows), {send, es, rows}, {which == b200collOpAllReduce ? recv : nullptr, es, 1}, st,
+                    [&](size_t done, size_t m) { return launch(kOffStage, kOffStage + kStageHalfBytes, out + done * es, m); });
 }
 
 }  // namespace b200coll

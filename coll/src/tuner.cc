@@ -91,13 +91,6 @@ static void load_rows() {
   for (const Row& r : kBuiltin) g_rows.push_back(r);
 }
 
-int tuner_blocks(b200collOp_t, b200collAlgo_t, size_t work_vecs, int max_ctas, int per_block) {
-  size_t b = (work_vecs + (size_t)per_block - 1) / (size_t)per_block;
-  if (b < 1) b = 1;
-  if (b > (size_t)max_ctas) b = (size_t)max_ctas;
-  return (int)b;
-}
-
 }  // namespace b200coll
 
 extern "C" {
